@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """Headline benchmark: MOG2 Mpixel/s at 1080p (BASELINE.json metric), one camera stream per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the timed headline path returned for the last frame of its last step (rank 0): the mask
+as DIR/foreground_mask.npy and the background image as DIR/background_image.npy, float32.  The synthetic input is seeded,
+so two builds run with the same arguments can be compared output for output.
 
 A "step" is one pass of the hot path over one batch of synthetic input: FRAMES_PER_STEP
 consecutive 1920x1080 BGR frames of one camera stream, advanced frame by frame (T = 1, the judged
@@ -314,6 +318,15 @@ def parity_check(ctx, my_c4_streams):
     return out
 
 
+def dump_outputs(outdir, arrays):
+    """Device arrays -> outdir/<name>.npy as float32 (the caller has synchronised the stream that wrote them)."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a.cpu().numpy().astype(np.float32))
+    log("bench.py: wrote %s to %s" % (", ".join(n + ".npy" for n in arrays), outdir))
+
+
 def headline(ctx, args):
     import tracking_b200 as tb
     from tracking_b200 import capi, synth
@@ -350,6 +363,8 @@ def headline(ctx, args):
     t_end = time.perf_counter()
     clocks = sampler.stop(t_begin, t_end) if ctx.rank == 0 else None
     launches = capi.kernel_launch_count() - launches0
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, {"foreground_mask": d_fg, "background_image": d_bg})
     ms = ev0.elapsed_time(ev1)
     ms_max = ctx.max_over_ranks([ms])[0]
     _, nm_host = bgs.export_state()
@@ -746,7 +761,11 @@ def main():
     ap.add_argument("--headline-only", action="store_true", help="profiling runs: only the headline workload")
     ap.add_argument("--frames-per-step", type=int, default=FRAMES_PER_STEP)
     ap.add_argument("--kernel-variant", type=int, default=0, help="0 production MOG2 kernel, 1 straight restatement (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline path's mask and background image of its last timed frame as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3:
         args.warmup = 3          # timing rule: W >= 3
     if args.impl == "reference":

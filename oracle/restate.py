@@ -34,9 +34,9 @@ class Mog2Params(C.Structure):
                 ("shadow_value", C.c_int), ("history", C.c_int)]
 
 
-def build_ref(reference="/root/reference"):
-    """Compile the reference's own DP-package models and Sigma-Delta library into oracle/_ref/libdp_ref.so (`make ref`) when the
-    reference tree is there; returns True if the library exists afterwards."""
+def build_ref(reference=os.environ.get("BGSB_REFERENCE_DIR", "/root/reference")):
+    """Compile the reference's own DP-package models and Sigma-Delta library into oracle/_ref/libdp_ref.so (`make ref`) when a
+    checkout of the original project is there ($BGSB_REFERENCE_DIR, else /root/reference); returns True if the library exists afterwards."""
     here = os.path.dirname(os.path.abspath(__file__))
     if os.path.exists(os.path.join(reference, "package_bgs", "dp", "ZivkovicAGMM.cpp")):
         subprocess.run(["make", "-C", here, "ref", "REFERENCE=" + reference], check=True, stdout=subprocess.DEVNULL)
@@ -248,7 +248,7 @@ class DPZivkovicAGMMBGS:
 
 
 class ReferenceDPZivkovic:
-    """The reference's own ZivkovicAGMM class, compiled from /root/reference by `make -C oracle ref`
+    """The reference's own ZivkovicAGMM class, compiled from the original project's sources by `make -C oracle ref`
     (oracle/_ref/libdp_ref.so).  Raises FileNotFoundError when that build is absent."""
 
     def __init__(self, w, h, threshold=25.0, alpha=0.001, gaussians=3):
@@ -429,7 +429,7 @@ class ReferenceSigmaDelta:
 
 class ReferenceDPSimple:
     """The reference's own AdaptiveMedianBGS / MeanBGS / WrenGA / PratiMediodBGS classes ("median" / "mean" / "wren" / "prati"), compiled from
-    /root/reference by `make -C oracle ref` (oracle/_ref/libdp_ref.so) and driven as their DP*BGS::process wrappers do.
+    the original project's sources by `make -C oracle ref` (oracle/_ref/libdp_ref.so) and driven as their DP*BGS::process wrappers do.
     Raises FileNotFoundError when that build is absent."""
 
     def __init__(self, kind, w, h, *params):

@@ -10,7 +10,7 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
-REFERENCE_DIR = "/root/reference"      # exists only in the build container, never on the GPU box
+REFERENCE_DIR = os.environ.get("BGSB_REFERENCE_DIR", "/root/reference")    # a checkout of the original project, if one is at hand
 
 
 def pytest_configure(config):
@@ -63,3 +63,15 @@ def stress_sequence(n=200, h=48, w=64, seed=7):
         f = pal[idx] + rng.integers(-2, 3, (h, w, 3))
         out.append(np.clip(f, 0, 255).astype(np.uint8))
     return out
+
+
+def drift_sequence(n, seed):
+    """83 x 57 noisy static scene (+-8) crossed by a drifting solid block of a random colour."""
+    rng = np.random.default_rng(seed)
+    base = rng.integers(0, 256, (57, 83, 3), dtype=np.uint8)
+    frames = []
+    for t in range(n):
+        f = np.clip(base.astype(np.int16) + rng.integers(-8, 9, base.shape), 0, 255).astype(np.uint8)
+        f[5 + t // 2:25 + t // 2, 10 + t:40 + t] = rng.integers(0, 256, 3)
+        frames.append(f)
+    return frames

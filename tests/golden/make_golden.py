@@ -1,12 +1,12 @@
 """Generates the golden fixtures of tests/golden/ from the reference's own data files.
 
-Run HERE (the container that has /root/reference and cv2 4.13); the outputs are committed and
-travel to the GPU box, which has neither /root/reference nor any need to decode video:
+Needs a checkout of the original project ($BGSB_REFERENCE_DIR, else /root/reference) and cv2 4.13; the outputs are
+committed, so the tests need neither the original project nor any video decoding:
 
-    python tests/golden/make_golden.py
+    BGSB_REFERENCE_DIR=<checkout of the original project> python tests/golden/make_golden.py
 
-Inputs  : /root/reference/dataset/video.avi  (320x176, 374 frames; BASELINE config 1)
-          /root/reference/frames/1..51.png   (320x240; read by Demo2.cpp:148-151)
+Inputs  : $BGSB_REFERENCE_DIR/dataset/video.avi  (320x176, 374 frames; BASELINE config 1)
+          $BGSB_REFERENCE_DIR/frames/1..51.png   (320x240; read by Demo2.cpp:148-151)
 Oracle  : oracle/cv2_chain.py -- the reference plugins replayed call-for-call on OpenCV 4.13
           (the library the plugins delegate all arithmetic to).
 Outputs : clips.npz     small crops of consecutive decoded frames (inputs for every test)
@@ -19,6 +19,7 @@ import hashlib
 import json
 import os
 import sys
+import zipfile
 
 import cv2
 import numpy as np
@@ -28,9 +29,18 @@ sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import cv2_chain as ref          # noqa: E402
 from oracle import blobdetect as ref_bd      # noqa: E402
 
-REF = "/root/reference"
+REF = os.environ.get("BGSB_REFERENCE_DIR", "/root/reference")
 NAMES = {0: "FrameDifferenceBGS", 1: "StaticFrameDifferenceBGS", 2: "WeightedMovingMeanBGS",
          3: "WeightedMovingVarianceBGS", 5: "MixtureOfGaussianV2BGS", 6: "AdaptiveBackgroundLearning"}
+
+
+def save_npz_lzma(path, **arrays):
+    """np.savez with LZMA members (np.load reads them): the clips stay under 1 MB, where savez_compressed's deflate
+    needs 1.3 MB."""
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_LZMA) as z:
+        for name, a in arrays.items():
+            with z.open(name + ".npy", "w") as f:
+                np.lib.format.write_array(f, a)
 
 
 def sha(arrs):
@@ -99,7 +109,7 @@ def main():
     # ragged sizes on purpose (190 = 5*32+30, 126; 150x101)
     video_clip = np.stack([f[24:150, 0:190] for f in video[56:88]])          # 32 x 126 x 190 x 3
     png_clip = np.stack([f[60:161, 80:230] for f in pngs[0:16]])             # 16 x 101 x 150 x 3
-    np.savez_compressed(os.path.join(HERE, "clips.npz"), video_clip=video_clip, png_clip=png_clip)
+    save_npz_lzma(os.path.join(HERE, "clips.npz"), video_clip=video_clip, png_clip=png_clip)
 
     golden = {"generator": "tests/golden/make_golden.py", "opencv": cv2.__version__,
               "decoder_note": "video.avi decoded by cv2.VideoCapture (FFMPEG) in the build container",

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Golden vectors for DPAdaptiveMedianBGS / DPMeanBGS / DPWrenGABGS / DPPratiMediodBGS / SigmaDeltaBGS from a build of the REFERENCE's own sources.
 
-Run in the build container (needs /root/reference):  make -C oracle ref && python tests/golden/make_golden_dp.py
+With a checkout of the original project:  make -C oracle ref REFERENCE=<checkout> && python tests/golden/make_golden_dp.py
 Writes tests/golden/golden_dp.json: SHA-256 of the plugins' output masks (the high-threshold masks of
 package_bgs/dp/{AdaptiveMedianBGS,MeanBGS,WrenGA,PratiMediodBGS}.cpp and package_bgs/bl/sdLaMa091.cpp, driven as the DP*BGS::process wrappers do) on the committed clips
 and on the deterministic stress sequence of tests/conftest.py, for several parameter sets.

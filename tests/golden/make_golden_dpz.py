@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Golden vectors for DPZivkovicAGMMBGS from a build of the REFERENCE's own sources.
 
-Run in the build container (needs /root/reference):  make -C oracle ref && python tests/golden/make_golden_dpz.py
+With a checkout of the original project:  make -C oracle ref REFERENCE=<checkout> && python tests/golden/make_golden_dpz.py
 Writes tests/golden/golden_dpz.json: SHA-256 of the plugin's output masks (the high-threshold mask of
 package_bgs/dp/ZivkovicAGMM.cpp, driven as DPZivkovicAGMMBGS::process does) on the committed clips and on the
 deterministic stress sequence of tests/conftest.py, for several parameter sets.

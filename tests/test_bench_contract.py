@@ -1,9 +1,12 @@
-"""bench.py contract checks that run without a GPU: the reference arm prints ONE JSON line with the agreed keys, and
-the product arm refuses to run without a CUDA device (no CPU fallback)."""
+"""bench.py contract checks: the reference arm prints ONE JSON line with the agreed keys, the product arm refuses to run
+without a CUDA device (no CPU fallback), and on a GPU --dump-outputs writes what the timed path computed."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -33,6 +36,30 @@ def test_reference_arm_other_ranks_exit_quietly():
     r = _run(["--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "1"],
              env={"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"})
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs_needs_the_product_arm(tmp_path):
+    r = _run(["--impl", "reference", "--steps", "1", "--warmup", "1", "--dump-outputs", str(tmp_path)])
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+    assert not os.listdir(tmp_path)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_frame(tmp_path, oracle):
+    """--dump-outputs after W warm-up and K timed steps of F frames == the oracle after (W + K) * F frames of the same
+    synthetic stream: the dump is the timed path's last output, and --steps sets how many steps ran."""
+    from tracking_b200 import synth
+    F, K, Wm = 3, 2, 3
+    r = _run(["--steps", str(K), "--warmup", str(Wm), "--frames-per-step", str(F), "--headline-only", "--no-e2e",
+              "--no-parity", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)])
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == K
+    fg, bg = np.load(tmp_path / "foreground_mask.npy"), np.load(tmp_path / "background_image.npy")
+    assert fg.dtype == bg.dtype == np.float32 and fg.shape == (1080, 1920) and bg.shape == (1080, 1920, 3)
+    o = oracle.MixtureOfGaussianV2BGS()
+    for t in range((Wm + K) * F):                  # the benchmark cycles 128 resident frames; fewer are used here
+        ofg, obg = o.process(oracle.synth_frame(1920, 1080, t, synth.SEED0))
+    assert np.array_equal(fg, ofg) and np.array_equal(bg, obg)
 
 
 def test_product_arm_needs_a_cuda_device():
