@@ -142,17 +142,6 @@ ccl_pack_kernel(const uint8_t *__restrict__ mask, unsigned *__restrict__ bits, i
     ccl_init_word(parent, word, y * w + k * 32);
 }
 
-// ---- launch 1 (bit-packed masks whose producer did not create the nodes) -----------------------------------------
-__global__ void __launch_bounds__(256)
-ccl_init_kernel(const __grid_constant__ CclArgs A)
-{
-    pdl_entry();
-    const int wi = blockIdx.x * blockDim.x + threadIdx.x;
-    if (wi >= A.nwords) return;
-    const int y = wi / A.wpr, k = wi - y * A.wpr;
-    ccl_init_word(A.parent + blockIdx.y * A.img_px, ccl_word(A.bits + blockIdx.y * A.img_words, y, k, A), y * A.w + k * 32);
-}
-
 template <bool DIAG>
 __device__ __forceinline__ void merge_class(int *parent, unsigned v, unsigned vl, unsigned vr, unsigned u,
                                             unsigned ul, unsigned ur, int base, int base_up, bool has_up)
@@ -814,8 +803,8 @@ int ccl_gather_tables(bgsb_ccl *c, int32_t *d_out, int rows, cudaStream_t stream
     return BGSB_OK;
 }
 
-// launches 2-4 (and the node init when the producer of the words did not do it)
-int ccl_label_bits(bgsb_ccl *c, const unsigned *d_bits, bool parents_ready, int w, int h, int nimages, int zero_border,
+// launches 2-4 (the producer of the words has created the nodes)
+int ccl_label_bits(bgsb_ccl *c, const unsigned *d_bits, int w, int h, int nimages, int zero_border,
                    int32_t *d_labels, cudaStream_t stream)
 {
     BGSB_REQUIRE(c && d_bits, "null");
@@ -845,10 +834,6 @@ int ccl_label_bits(bgsb_ccl *c, const unsigned *d_bits, bool parents_ready, int 
     c->table_images = nimages;
     c->dirty = true;
     const dim3 block(256);
-    if (!parents_ready) {
-        launch_pdl(ccl_init_kernel, dim3((A.nwords + 255) / 256, nimages), block, 0, stream, A);
-        BGSB_LAUNCH_CHECK();
-    }
     // Words per thread: 1 for a single image (254 CTAs at 1080p fill the SMs), 4 for batches too big for one wave of
     // one-word CTAs.  (16 words per thread was measured and removed: a sixteenth of the CTAs, but the per-word work of a
     // thread is serial -- 64 masks 166 -> 284 us, 8 masks 44 -> 117 us.)
@@ -987,7 +972,7 @@ int bgsb_ccl_label_batch_dev(bgsb_ccl *c, const uint8_t *d_masks, int w, int h, 
     launch_pdl(ccl_pack_kernel, grid, dim3(256), 0, stream, d_masks, c->d_bits, c->d_parent, w, h, wpr, zero_border,
                (size_t)w * h, (size_t)nwords);
     BGSB_LAUNCH_CHECK();
-    int rc = ccl_label_bits(c, c->d_bits, true, w, h, nimages, 0, d_labels, stream);
+    int rc = ccl_label_bits(c, c->d_bits, w, h, nimages, 0, d_labels, stream);
     if (rc) return rc;
     c->last_mask = d_masks; c->last_bits = nullptr;
     return BGSB_OK;

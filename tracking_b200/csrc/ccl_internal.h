@@ -45,9 +45,9 @@ namespace bgsb {
 
 // Label `nimages` bit-packed masks ([nimages][h][wpr] words, bit i of word k = pixel 32k+i of the row; bits beyond the
 // row end must be zero).  zero_border: the 1-px frame counts as background (applied on the fly, the words are not
-// modified).  parents_ready: the producer of the words has already made every run start its own union-find root
-// (ccl_init_word); otherwise an init launch does it.
-int ccl_label_bits(bgsb_ccl *c, const unsigned *d_bits, bool parents_ready, int w, int h, int nimages, int zero_border,
+// modified).  The producer of the words must already have made every run start its own union-find root
+// (ccl_init_word: the pack kernel and the morphology kernel do).
+int ccl_label_bits(bgsb_ccl *c, const unsigned *d_bits, int w, int h, int nimages, int zero_border,
                    int32_t *d_labels, cudaStream_t stream);
 
 // [nimages][(rows + 1) * 8] ints: per image {count, 0 x 7} then `rows` decoded bgsb_component rows (the first `rows`

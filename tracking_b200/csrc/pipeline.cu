@@ -203,12 +203,12 @@ int bgsb_pipeline_process_dev(bgsb_pipeline *p, const uint8_t *d_frames, int w, 
         io.in_bits = p->d_raw[slot]; io.out_bits = p->d_clean;
         rc = launch_morph_chain_io(io, w, h, S, p->ops, p->nops, cs);
         if (rc) return rc;
-        rc = ccl_label_bits(p->ccl, p->d_clean, true, w, h, S, p->zero_border, d_labels, cs);
+        rc = ccl_label_bits(p->ccl, p->d_clean, w, h, S, p->zero_border, d_labels, cs);
     } else if (p->total_iters > 0) {
         io.in_bytes = p->d_fg[slot]; io.out_bits = p->d_clean;
         rc = launch_morph_chain_io(io, w, h, S, p->ops, p->nops, cs);
         if (rc) return rc;
-        rc = ccl_label_bits(p->ccl, p->d_clean, true, w, h, S, p->zero_border, d_labels, cs);
+        rc = ccl_label_bits(p->ccl, p->d_clean, w, h, S, p->zero_border, d_labels, cs);
     } else {
         // no chain on a byte mask: the labeller's own pack step applies DetectNewBlob's threshold (> 128)
         if (d_mask) BGSB_CUDA(cudaMemcpyAsync(d_mask, p->d_fg[slot], (size_t)S * w * h, cudaMemcpyDeviceToDevice, cs));
