@@ -103,6 +103,8 @@ BGSB_API int bgsb_reset(bgsb_ctx *ctx);
 /* Parameters carry the reference's XML key names (saveConfig/loadConfig of each plugin):
  *   all      : "enableThreshold" (1), "threshold" (15)
  *   MOG2     : "alpha" (0.05)             MixtureOfGaussianV2BGS.cpp:92-95
+ *              (as cv::BackgroundSubtractorMOG2::apply: alpha >= 1 re-initialises the model before every frame, which then
+ *              learns at 1/min(2, history); after it, alpha < 0 counts its automatic rate from that frame again)
  *   ABL      : "alpha" (0.05), "limit" (-1; only -1 updates the model, .cpp:52)
  *   DPZivkovicAGMM : "threshold" (25.0), "alpha" (0.001), "gaussians" (3, at most 5)   DPZivkovicAGMMBGS.cpp:86-100
  *              (latched at the first frame like the reference's params hand-over, .cpp:58-65: a later change takes
@@ -114,7 +116,7 @@ BGSB_API int bgsb_reset(bgsb_ctx *ctx);
  * (MixtureOfGaussianV2BGS.h:30): "history" 500, "nmixtures" 5 (fixed), "varThreshold" 16,
  * "varThresholdGen" 9, "backgroundRatio" 0.9, "varInit" 15, "varMin" 4, "varMax" 75,
  * "complexityReductionThreshold" 0.05, "detectShadows" 1, "shadowValue" 127,
- * "shadowThreshold" 0.5; and "grayVariant": 0 = OpenCV 4.x BGR2GRAY constants, 1 = 2.4.x;
+ * "shadowThreshold" 0.5 (varMin / varMax given in the wrong order are swapped, as OpenCV does); and "grayVariant": 0 = OpenCV 4.x BGR2GRAY constants, 1 = 2.4.x;
  * "kernelVariant" (MOG2): 0 = production kernels, 1 = straight restatement kernel (identical results, kept for
  * A/B measurements).  (8, 9 = timing instruments with WRONG results exist only in a library built with
  * -DBGSB_INSTRUMENT for tools/floor_probe.py; the shipped library rejects them);
@@ -323,6 +325,10 @@ BGSB_API int bgsb_pipeline_set_param(bgsb_pipeline *p, const char *key, double v
  *   d_bg     [nstreams][h][w][3] the plugin's background image
  *   d_labels [nstreams][h][w]    canonical labels of the 8-connected components (int32, 0 = background)
  * *valid = 0 while the plugin has no mask yet (FD frame 0, WMV frames 0-1): nothing was labelled.
+ * With the plugin's "enableThreshold" 0 and a chain, the reference erodes / dilates the raw grey-level mask and
+ * DetectNewBlob keeps what is > 128 afterwards: the pipeline labels exactly those pixels (it thresholds before the chain,
+ * which commutes with erode / dilate), but it has no grey-level cleaned mask, so d_mask must be NULL (BGSB_ERR_ARG
+ * otherwise) and bgsb_pipeline_rect_moments refuses that frame.  The stream pool inherits both.
  * Asynchronous.  The plugin kernel runs on `stream`; clean-up and labelling run on a stream of the pipeline behind
  * it, so that they overlap whatever the caller enqueues next on `stream` (normally the next frame's plugin kernel).
  * `stream` is made to wait for them only when d_mask or d_labels were given; otherwise the component tables (which
@@ -338,7 +344,8 @@ BGSB_API int bgsb_pipeline_components(bgsb_pipeline *p, int stream_index, bgsb_c
  * by the first rows_per_stream components (raster order) as bgsb_component rows.  Asynchronous: `stream` (any stream of
  * the device, e.g. the one a download is enqueued on next) waits for the buffer to be complete. */
 BGSB_API int bgsb_pipeline_tables_dev(bgsb_pipeline *p, int32_t *d_out, int rows_per_stream, void *stream);
-/* cvMoments(pFGMask[R], 0) sums on that stream's cleaned mask, as bgsb_ccl_rect_moments. */
+/* cvMoments(pFGMask[R], 0) sums on that stream's cleaned mask, as bgsb_ccl_rect_moments.  BGSB_ERR_ARG when the last
+ * frame had the plugin's threshold off and a chain (see bgsb_pipeline_process_dev). */
 BGSB_API int bgsb_pipeline_rect_moments(bgsb_pipeline *p, int stream_index, const int32_t *rects_xywh, int nrects,
                                         uint64_t *out);
 

@@ -525,7 +525,8 @@ ORC_API void orc_mog2_default_params(orc_mog2_params *p)
 }
 
 /* learning rate rule of operator(): ++nframes;
- * lr = (alpha >= 0 && nframes > 1) ? alpha : 1./min(2*nframes, history) */
+ * lr = (alpha >= 0 && nframes > 1) ? alpha : 1./min(2*nframes, history).
+ * alpha >= 1 re-initialises the model first (needToInitialize, nframes = 0): the caller then passes nframes 1. */
 ORC_API double orc_mog2_learning_rate(double alpha, int nframes_after_increment, int history)
 {
     if (alpha >= 0 && nframes_after_increment > 1) return alpha;
@@ -569,6 +570,9 @@ ORC_API void orc_mog2_apply(const uint8_t *in, int npx, double lr, const orc_mog
     const int K = P->K;
     const float alphaT = (float)lr, alpha1 = 1.f - alphaT;
     const float prune = (float)(-lr * (double)P->CT);   /* float prune = -learningRate*fCT (fCT float, product in double) */
+    /* MOG2Invoker: varMin = min(_varMin, _varMax), varMax = max(_varMin, _varMax) */
+    const float varMin = P->varMin < P->varMax ? P->varMin : P->varMax;
+    const float varMax = P->varMin < P->varMax ? P->varMax : P->varMin;
     for (int i = 0; i < npx; i++) {
         float *gmm = gmm_all + (size_t)i * K * 2;
         float *mean = mean_all + (size_t)i * K * 3;
@@ -591,8 +595,8 @@ ORC_API void orc_mog2_apply(const uint8_t *in, int npx, double lr, const orc_mog
                     float k = alphaT / w;
                     mu[0] -= k * dD0; mu[1] -= k * dD1; mu[2] -= k * dD2;
                     float vn = var + k * (dist2 - var);
-                    vn = vn > P->varMin ? vn : P->varMin;       /* MAX(varnew, fVarMin) */
-                    vn = vn < P->varMax ? vn : P->varMax;       /* MIN(varnew, fVarMax) */
+                    vn = vn > varMin ? vn : varMin;             /* MAX(varnew, varMin) */
+                    vn = vn < varMax ? vn : varMax;             /* MIN(varnew, varMax) */
                     gmm[2 * m + 1] = vn;
                     for (int j = m; j > 0; j--) {
                         if (w < gmm[2 * (j - 1)]) break;

@@ -224,9 +224,21 @@ class MixtureOfGaussianV2BGS:
     """package_bgs/MixtureOfGaussianV2BGS.cpp:29-74.  `cv::BackgroundSubtractorMOG2 mog;`
     default-constructed (history 500, varThreshold 16, shadows on) -> cv2.createBackgroundSubtractorMOG2()."""
 
-    def __init__(self, alpha=0.05, enableThreshold=True, threshold=15):
+    # bgsb_set_param keys of the model's own parameters -> cv::BackgroundSubtractorMOG2 setters
+    SETTERS = {"history": "setHistory", "varThreshold": "setVarThreshold", "varThresholdGen": "setVarThresholdGen",
+               "backgroundRatio": "setBackgroundRatio", "varInit": "setVarInit", "varMin": "setVarMin", "varMax": "setVarMax",
+               "complexityReductionThreshold": "setComplexityReductionThreshold", "shadowThreshold": "setShadowThreshold",
+               "detectShadows": "setDetectShadows", "shadowValue": "setShadowValue"}
+
+    def __init__(self, alpha=0.05, enableThreshold=True, threshold=15, **model):
         self.alpha, self.enableThreshold, self.threshold = alpha, enableThreshold, threshold
         self.mog = cv2.createBackgroundSubtractorMOG2()
+        for k, v in model.items():
+            if k == "detectShadows":
+                v = bool(v)
+            elif k in ("history", "shadowValue"):
+                v = int(v)
+            getattr(self.mog, self.SETTERS[k])(v)
 
     def process(self, img):
         if img is None or img.size == 0:

@@ -489,10 +489,18 @@ class WeightedMovingVarianceBGS:
 class MixtureOfGaussianV2BGS:
     """MOG2 wrapper (package_bgs/MixtureOfGaussianV2BGS.cpp:56-62) over orc_mog2_*."""
 
-    def __init__(self, alpha=0.05, enableThreshold=True, threshold=15):
+    # bgsb_set_param keys of the model's own parameters -> orc_mog2_params fields
+    KEYS = {"varThreshold": "Tb", "varThresholdGen": "Tg", "backgroundRatio": "TB", "varInit": "varInit", "varMin": "varMin",
+            "varMax": "varMax", "complexityReductionThreshold": "CT", "shadowThreshold": "tau", "detectShadows": "detect_shadows",
+            "shadowValue": "shadow_value", "history": "history"}
+
+    def __init__(self, alpha=0.05, enableThreshold=True, threshold=15, **model):
         self.alpha, self.enableThreshold, self.threshold = alpha, enableThreshold, threshold
         self.params = Mog2Params()
         lib().orc_mog2_default_params(C.byref(self.params))
+        for k, v in model.items():
+            field = self.KEYS[k]
+            setattr(self.params, field, type(getattr(self.params, field))(v))
         self.nframes = 0
         self.shape = None
 
@@ -509,7 +517,7 @@ class MixtureOfGaussianV2BGS:
         if img is None or img.size == 0:
             return None, None
         img = _dense(img)
-        if self.shape != img.shape[:2]:          # operator(): re-initialise on size change
+        if self.shape != img.shape[:2] or self.alpha >= 1:   # apply(): needToInitialize on a size change or learningRate >= 1
             self._init(img.shape[:2])
         self.nframes += 1
         lr = lib().orc_mog2_learning_rate(float(self.alpha), self.nframes, self.params.history)

@@ -319,6 +319,9 @@ ROWS = [
     Row("mog2_t1_group_odd_px", MOG2, {"mog2_t1_kernel"}, h=33, w=41, S=3, skip=1),
     Row("mog2_fused_T8_all+1", MOG2, {"mog2_fused_kernel"}, h=33, w=41, T=8, n=3, frames=1, fg=1, bgo=1, skip=1),
     Row("mog2_restatement_variant1", MOG2, {"mog2_kernel"}, h=33, w=41, kw=dict(kernelVariant=1), skip=1),
+    # alpha >= 1 re-initialises the model on every frame: batches run one frame (and one stream) per launch
+    Row("mog2_reinit_T8_per_frame", MOG2, {"mog2_t1_kernel"}, h=33, w=41, T=8, n=3, kw=dict(alpha=1.5), skip=1),
+    Row("mog2_reinit_T8_group_per_frame", MOG2, {"mog2_t1_kernel"}, h=33, w=41, S=2, T=8, n=3, kw=dict(alpha=1.0), skip=1),
 ]
 
 # DPMean / DPWrenGA / DPPratiMediod / DPZivkovicAGMM: frame and mask pointers off the 4-byte grid (the v12 / v4 word

@@ -7,25 +7,9 @@ import numpy as np
 import pytest
 
 from conftest import stress_sequence
+from param_draws import scene
 
 pytestmark = pytest.mark.gpu
-
-
-def scene(rng, n, h, w):
-    """noisy background with drifting brightness, a few moving bright / dark blobs, occasional palette flips"""
-    base = rng.integers(30, 200, (h, w, 3)).astype(np.int16)
-    yy, xx = np.mgrid[0:h, 0:w]
-    out = []
-    for t in range(n):
-        f = base + rng.integers(-4, 5, (h, w, 3)) + int(6 * np.sin(t / 3.0))
-        for b in range(3):
-            cy, cx = (7 * t + 31 * b) % h, (11 * t + 17 * b) % w
-            m = (yy - cy) ** 2 + (xx - cx) ** 2 < (5 + 2 * b) ** 2
-            f[m] = (250, 10 + 60 * b, 128) if b != 1 else f[m] // 2            # b == 1: a shadow-like darker copy
-        if t % 9 == 8:
-            f[:, : w // 3] = base[:, : w // 3][..., ::-1]
-        out.append(np.clip(f, 0, 255).astype(np.uint8))
-    return out
 
 
 MOG2_KEYS = {"varThreshold": "Tb", "varThresholdGen": "Tg", "backgroundRatio": "TB", "varInit": "varInit", "varMin": "varMin",

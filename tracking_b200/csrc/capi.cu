@@ -73,6 +73,8 @@ struct bgsb_ctx {
     int w = 0, h = 0, npx = 0;
     size_t pstride = 0;
     int64_t nframes = 0;
+    int64_t mog2_epoch = 0;    // MOG2: the frame (counted in nframes) that last re-initialised the model (learningRate >= 1);
+                               // the model's own frame counter, which drives the automatic learning rate, is nframes - mog2_epoch
     // device state
     float *d_state = nullptr;
     uint8_t *d_nmodes = nullptr;
@@ -153,7 +155,7 @@ static void free_buffers(bgsb_ctx *c)
     cudaFree(c->d_fan); c->d_fan = nullptr; c->d_fan_bytes = 0;
     cudaFree(c->d_prati); c->d_prati = nullptr; c->prati_bytes = 0; c->prati_n = c->prati_pos = 0;
     c->w = c->h = c->npx = 0; c->pstride = 0;
-    c->nframes = 0; c->have_hist = 0; c->ring_pos = 0;
+    c->nframes = 0; c->mog2_epoch = 0; c->have_hist = 0; c->ring_pos = 0;
 }
 
 // (Re)allocate model state for a geometry.  The reference discovers the frame size on the first
@@ -279,14 +281,26 @@ static int launch_range(bgsb_ctx *c, const uint8_t *d_frames, int T, uint8_t *d_
 {
     if (c->algo == BGSB_ALGO_MOG2) {
         BGSB_REQUIRE(T <= MOG2_TMAX, "temporal batch too long (max 32)");
+        // learningRate >= 1: cv::BackgroundSubtractorMOG2::apply re-initialises the model before every such frame
+        // (needToInitialize), so each frame starts from an empty model with nframes = 1.  No frame can reuse another's
+        // state: a batch runs one frame per launch, and a group one stream per launch too (a launch's streams sit L.T
+        // frames apart in the batch layouts).
+        const bool reinit = c->alpha >= 1;
         // Short batches of one stream run frame by frame: the T == 1 kernel costs less per frame than the
         // temporal-fusion kernel's fixed state load/store until about six frames share it (profiles/).
-        const bool per_frame = T > 1 && T < 6 && c->nstreams == 1 && c->mog2_variant == 0;
+        const bool per_frame = T > 1 && ((T < 6 && c->nstreams == 1 && c->mog2_variant == 0) || reinit);
+        const bool per_stream = per_frame && c->nstreams > 1;
         const int nlaunch = per_frame ? T : 1, Tl = per_frame ? 1 : T;
+        const int nsplit = per_stream ? c->nstreams : 1, Sl = per_stream ? 1 : c->nstreams;
+        // frames the model has seen since it was last (re)initialised (OpenCV's nframes)
+        const int64_t seen = c->nframes - c->mog2_epoch;
+        // MOG2Invoker: varMin = min(_varMin, _varMax), varMax = max(_varMin, _varMax)
+        const float vmin = std::min(c->varMin, c->varMax), vmax = std::max(c->varMin, c->varMax);
+        for (int s = 0; s < nsplit; s++)
         for (int i = 0; i < nlaunch; i++) {
             Mog2Launch L;
             memset(&L, 0, sizeof(L));
-            const size_t f0 = (size_t)i * c->npx;                  // first pixel of frame i in the batch buffers
+            const size_t f0 = ((size_t)s * T + i) * c->npx;        // first pixel of frame i of stream s in the batch buffers
             L.frames = d_frames + (f0 + p0) * 3; L.fg = d_fg ? d_fg + f0 + p0 : nullptr;
             L.bg = nullptr;
             if (d_bits) {                                  // whole single frames on the production kernel only (ctx_process_frame)
@@ -295,29 +309,31 @@ static int launch_range(bgsb_ctx *c, const uint8_t *d_frames, int T, uint8_t *d_
             if (d_bg) {
                 if (!per_frame) L.bg = d_bg + p0 * 3;
                 else if (!bg_last_only) L.bg = d_bg + (f0 + p0) * 3;
-                else if (i == T - 1) L.bg = d_bg + p0 * 3;
+                else if (i == T - 1) L.bg = d_bg + ((size_t)s * c->npx + p0) * 3;
             }
-            L.state = c->d_state + p0 * MOG2_PLANES; L.nmodes = c->d_nmodes + p0; L.pstride = c->pstride;   // p0 % 64 == 0
+            L.state = c->d_state + ((size_t)s * c->pstride + p0) * MOG2_PLANES;   // p0 % 64 == 0
+            L.nmodes = c->d_nmodes + (size_t)s * c->pstride + p0; L.pstride = c->pstride;
             L.npx = pcount; L.T = Tl; L.bg_last_only = per_frame ? 0 : bg_last_only;
-            L.fresh = (c->nframes + i == 0);
+            L.fresh = reinit || seen + i == 0;
             L.fast_ok = 1;
             L.one = 1.f;
             L.enable_thr = c->enable_thr; L.thr = c->thr;
             L.detect_shadows = c->detect_shadows; L.shadow_value = c->shadow_value;
-            L.Tb = c->Tb; L.Tg = c->Tg; L.TB = c->TB; L.varInit = c->varInit; L.varMin = c->varMin;
-            L.varMax = c->varMax; L.tau = c->tau;
+            L.Tb = c->Tb; L.Tg = c->Tg; L.TB = c->TB; L.varInit = c->varInit; L.varMin = vmin;
+            L.varMax = vmax; L.tau = c->tau;
             for (int t = 0; t < Tl; t++) {
                 // operator(): ++nframes; learningRate = alpha>=0 && nframes>1 ? alpha : 1./min(2*nframes, history)
-                int64_t nf = c->nframes + i + t + 1;
+                int64_t nf = reinit ? 1 : seen + i + t + 1;
                 double lr = (c->alpha >= 0 && nf > 1) ? c->alpha : 1. / (double)std::min<int64_t>(2 * nf, c->history);
                 L.alphaT[t] = (float)lr;
                 L.alpha1[t] = 1.f - L.alphaT[t];
                 L.prune[t] = (float)(-lr * (double)c->CT);
                 if (!(L.alphaT[t] >= 1e-4f && L.alphaT[t] <= 1.f)) L.fast_ok = 0;
             }
-            int rc = launch_mog2(L, c->nstreams, c->mog2_variant, stream);
+            int rc = launch_mog2(L, Sl, c->mog2_variant, stream);
             if (rc) return rc;
         }
+        if (reinit) c->mog2_epoch = c->nframes + T - 1;  // the last frame of the batch re-initialised the model
     } else if (c->algo == BGSB_ALGO_DP_ZIVKOVIC_AGMM) {
         for (int t = 0; t < T; t++) {
             DpzLaunch L;
@@ -679,7 +695,7 @@ int bgsb_reset(bgsb_ctx *c)
     BGSB_REQUIRE(c, "null ctx");
     int rc = drain(c);
     if (rc) return rc;
-    c->nframes = 0; c->have_hist = 0; c->asbl_counter = 0;
+    c->nframes = 0; c->mog2_epoch = 0; c->have_hist = 0; c->asbl_counter = 0;
     c->hist_ptr[0] = c->hist_ptr[1] = nullptr;
     return BGSB_OK;
 }
@@ -1210,7 +1226,7 @@ int bgsb_mog2_import_state(bgsb_ctx *c, int si, int w, int h, int64_t nframes, c
                                       cudaMemcpyHostToDevice));
     }
     BGSB_CUDA(cudaMemcpy(c->d_nmodes + (size_t)si * c->pstride, nmodes, c->npx, cudaMemcpyHostToDevice));
-    c->nframes = nframes;
+    c->nframes = nframes; c->mog2_epoch = 0;
     return BGSB_OK;
 }
 

@@ -893,6 +893,20 @@ int ccl_label_bits(bgsb_ccl *c, const unsigned *d_bits, int w, int h, int nimage
     return BGSB_OK;
 }
 
+int ccl_pack_bytes(bgsb_ccl *c, const uint8_t *d_masks, unsigned *d_bits, int w, int h, int nimages, cudaStream_t stream)
+{
+    BGSB_REQUIRE(c && d_masks && d_bits, "null");
+    BGSB_REQUIRE(w > 0 && h > 0 && w <= c->max_w && h <= c->max_h, "image larger than the labeller was created for");
+    BGSB_REQUIRE(nimages >= 1 && nimages <= c->max_images, "more images than the labeller was created for");
+    BGSB_CUDA(cudaSetDevice(c->device));
+    const int wpr = (w + 31) / 32, nwords = wpr * h;
+    // (the nodes it creates are replaced by those of the morphology kernel that reads the words)
+    launch_pdl(ccl_pack_kernel, dim3((nwords + 255) / 256, nimages), dim3(256), 0, stream, d_masks, d_bits, c->d_parent, w, h,
+               wpr, 0, (size_t)w * h, (size_t)nwords);
+    BGSB_LAUNCH_CHECK();
+    return BGSB_OK;
+}
+
 }  // namespace bgsb
 
 using namespace bgsb;

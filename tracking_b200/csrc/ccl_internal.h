@@ -50,6 +50,10 @@ namespace bgsb {
 int ccl_label_bits(bgsb_ccl *c, const unsigned *d_bits, int w, int h, int nimages, int zero_border,
                    int32_t *d_labels, cudaStream_t stream);
 
+// Pack [nimages][h][w] byte masks into [nimages][h][wpr] words with DetectNewBlob's threshold (a bit per byte > 128),
+// frame kept, so that the words can go through the morphology kernel before labelling.
+int ccl_pack_bytes(bgsb_ccl *c, const uint8_t *d_masks, unsigned *d_bits, int w, int h, int nimages, cudaStream_t stream);
+
 // [nimages][(rows + 1) * 8] ints: per image {count, 0 x 7} then `rows` decoded bgsb_component rows (the first `rows`
 // components in raster order); asynchronous on `stream`, which must be the stream of the labelling call.
 int ccl_gather_tables(bgsb_ccl *c, int32_t *d_out, int rows, cudaStream_t stream);

@@ -41,6 +41,7 @@ struct bgsb_pipeline {
     unsigned *d_clean = nullptr;                        // ... after the chain
     uint8_t *d_fg[NSLOT] = {};                          // [S][h][w] byte masks of plugins that cannot emit bits
     bool labelled = false;
+    bool raw_chain = false;                             // the last labelled frame: threshold off, chain on (no moments)
     // Clean-up + labelling of frame t run on the pipeline's own high-priority stream, so that they overlap the plugin
     // kernel of frame t+1 (their launches are latency-bound and leave the SMs almost empty): the caller's stream only
     // waits for them when it has to (device outputs requested, or bgsb_pipeline_join_dev).
@@ -171,6 +172,16 @@ int bgsb_pipeline_process_dev(bgsb_pipeline *p, const uint8_t *d_frames, int w, 
     // raw mask values (shadow = 127), so that combination keeps the byte mask.
     double thr_on = 1.;
     (void)bgsb_get_param(p->bgs, "enableThreshold", &thr_on);
+    // With the threshold off and a chain, the reference erodes / dilates the raw grey-level mask and DetectNewBlob then
+    // keeps the pixels > 128.  Thresholding commutes with erode / dilate (min / max), so packing "> 128" BEFORE the chain
+    // labels the same pixels; the cleaned grey-level mask and its moments would need grey-level morphology, so they are
+    // refused in that combination.
+    const bool raw_chain = thr_on == 0. && p->total_iters > 0;
+    if (raw_chain && d_mask) {
+        set_error("bgsb_pipeline_process_dev: no cleaned mask with enableThreshold = 0 and an erode / dilate chain (the "
+                  "reference's is grey-level); pass d_mask = NULL");
+        return BGSB_ERR_ARG;
+    }
     const bool pack = ctx_can_pack(p->bgs) && (p->total_iters > 0 || thr_on != 0.);
     const int slot = (int)(p->nframe % bgsb_pipeline::NSLOT);
     if (!pack && !p->d_fg[slot]) BGSB_CUDA(cudaMalloc(&p->d_fg[slot], (size_t)S * w * h));
@@ -178,10 +189,11 @@ int bgsb_pipeline_process_dev(bgsb_pipeline *p, const uint8_t *d_frames, int w, 
     if (p->chain_used[slot]) BGSB_CUDA(cudaStreamWaitEvent(stream, p->ev_chain[slot], 0));
     int packed = 0, fv = 0, bv = 0;
     if (pack) {
-        // the plugin kernel ORs its foreground bits into zeroed rows; a pixel counts when its mask byte would be non-zero
-        // (what the morphology reads) or, without a chain, > 128 (what cvThreshold(128) in DetectNewBlob keeps)
+        // the plugin kernel ORs its foreground bits into zeroed rows; a pixel counts when its mask byte is > 128 (what
+        // cvThreshold(128) in DetectNewBlob keeps; on a thresholded {0,255} mask the same as non-zero, which is what the
+        // morphology reads)
         // (the rows are zero: cleared at allocation and, after every use, behind the chain that read them)
-        rc = ctx_process_frame(p->bgs, d_frames, w, h, nullptr, d_bg, p->d_raw[slot], p->total_iters > 0 ? 0 : 128, &packed, &fv, &bv, stream);
+        rc = ctx_process_frame(p->bgs, d_frames, w, h, nullptr, d_bg, p->d_raw[slot], 128, &packed, &fv, &bv, stream);
     } else {
         rc = ctx_process_frame(p->bgs, d_frames, w, h, p->d_fg[slot], d_bg, nullptr, 0, &packed, &fv, &bv, stream);
     }
@@ -200,6 +212,14 @@ int bgsb_pipeline_process_dev(bgsb_pipeline *p, const uint8_t *d_frames, int w, 
     if (packed) {
         // (an empty chain still goes through the kernel: it copies the rows to d_clean -- the plugin's rows are cleared
         // below for their next use -- and creates the labeller's nodes)
+        io.in_bits = p->d_raw[slot]; io.out_bits = p->d_clean;
+        rc = launch_morph_chain_io(io, w, h, S, p->ops, p->nops, cs);
+        if (rc) return rc;
+        rc = ccl_label_bits(p->ccl, p->d_clean, w, h, S, p->zero_border, d_labels, cs);
+    } else if (raw_chain) {
+        // raw grey-level mask: DetectNewBlob's threshold first (the labeller's pack step), then the chain on the words
+        rc = ccl_pack_bytes(p->ccl, p->d_fg[slot], p->d_raw[slot], w, h, S, cs);
+        if (rc) return rc;
         io.in_bits = p->d_raw[slot]; io.out_bits = p->d_clean;
         rc = launch_morph_chain_io(io, w, h, S, p->ops, p->nops, cs);
         if (rc) return rc;
@@ -223,6 +243,7 @@ int bgsb_pipeline_process_dev(bgsb_pipeline *p, const uint8_t *d_frames, int w, 
     // chain running beside whatever the caller enqueues next (the next frame's plugin kernel)
     if (d_mask || d_labels) BGSB_CUDA(cudaStreamWaitEvent(stream, p->ev_chain[slot], 0));
     p->labelled = true;
+    p->raw_chain = raw_chain;
     if (valid) *valid = 1;
     return BGSB_OK;
 }
@@ -258,6 +279,11 @@ int bgsb_pipeline_rect_moments(bgsb_pipeline *p, int stream_index, const int32_t
 {
     BGSB_REQUIRE(p && out, "null");
     if (!p->labelled) { set_error("bgsb_pipeline_rect_moments: no frame has produced a mask yet"); return BGSB_ERR_STATE; }
+    if (p->raw_chain) {
+        set_error("bgsb_pipeline_rect_moments: with enableThreshold = 0 and an erode / dilate chain the reference weighs the "
+                  "grey-level cleaned mask, which the pipeline does not compute");
+        return BGSB_ERR_ARG;
+    }
     return bgsb_ccl_rect_moments_of(p->ccl, stream_index, rects, nrects, out);
 }
 
