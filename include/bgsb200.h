@@ -348,6 +348,23 @@ BGSB_API int bgsb_pipeline_tables_dev(bgsb_pipeline *p, int32_t *d_out, int rows
  * frame had the plugin's threshold off and a chain (see bgsb_pipeline_process_dev). */
 BGSB_API int bgsb_pipeline_rect_moments(bgsb_pipeline *p, int stream_index, const int32_t *rects_xywh, int nrects,
                                         uint64_t *out);
+/* CvBlobDetectorCC::DetectNewBlob for every stream of the last frame, on the labelling the pipeline already ran:
+ * bds[s] is stream s's detector (its own lists, tracks and parameters; the same object works with
+ * bgsb_blobdetector_detect[_dev] and bgsb_pool_detect), and the results are those of bgsb_blobdetector_detect on the
+ * stream's cleaned mask.  One download of all tables, the clustering on the host, ONE moments launch for all streams
+ * and one download of the sums: two synchronisations per call whatever nstreams is.
+ *   bds[S]         : distinct detectors whose "zeroBorder" is the pipeline's (the masks were labelled with it)
+ *   old_blobs[S]   : per stream the tracked blobs (n_old[s] of them; an entry may be NULL when n_old[s] == 0);
+ *                    old_blobs == NULL: no stream has any (n_old may then be NULL too)
+ *   new_blobs[S]   : stream s's new blob when result[s] == 1
+ *   frame_blobs    : nullable, [S][10]: stream s's sorted top-10 (m_pBlobLists[0]), n_frame[s] of them (nullable)
+ *   status[S]      : BGSB_OK per stream
+ * BGSB_ERR_STATE when the last frame produced no mask (plugin warm-up); BGSB_ERR_ARG for a NULL or repeated detector, a
+ * "zeroBorder" mismatch, or the threshold-off-with-chain combination (see bgsb_pipeline_process_dev).  On an error no
+ * detector advances. */
+BGSB_API int bgsb_pipeline_detect(bgsb_pipeline *p, bgsb_blobdetector *const *bds, const bgsb_blob *const *old_blobs,
+                                  const int *n_old, bgsb_blob *new_blobs, int *result, bgsb_blob *frame_blobs,
+                                  int *n_frame, int *status);
 
 /* ---------------------------------------------------------------------------------------
  * Stream pool: N camera streams of one geometry over the GPUs of this process (SURVEY 8e; BASELINE configs 4 / 5).
@@ -356,26 +373,41 @@ BGSB_API int bgsb_pipeline_rect_moments(bgsb_pipeline *p, int stream_index, cons
  * thread, one bgsb_pipeline over its streams, and `ring` slots of page-locked frame / mask / table buffers on three CUDA
  * streams, so that slot k+1 uploads while slot k computes and slot k-1 downloads.  Streams never exchange data.
  *   capture side : write frame t of stream s into bgsb_pool_frame_buffer(pool, s, t % ring)   (h*w*3 bytes, dense BGR)
- *   bgsb_pool_submit(pool, slot, want_masks) : every stream's frame of that slot is ready; returns at once
+ *   bgsb_pool_submit(pool, slot, flags)      : every stream's frame of that slot is ready; returns at once
  *   bgsb_pool_wait(pool, slot, &valid)       : that slot's results are on the host; valid = 0 while the plugin warms up
  *   bgsb_pool_mask / bgsb_pool_components    : the cleaned {0,255} mask (if asked for) and the component table
- *                                              (first 256 components in raster order) of one stream
- * A slot may be refilled and resubmitted once it has been waited for.  One thread drives submit / wait.
+ *                                              (first "tableRows" components in raster order) of one stream
+ *   bgsb_pool_detect(pool, slot, ...)        : DetectNewBlob for every stream of the slot (submitted with
+ *                                              BGSB_POOL_DETECT), between its wait and its next submit
+ * A slot may be refilled and resubmitted once it has been waited for.  One thread drives submit / wait / detect.
+ * Submit flags: BGSB_POOL_MASKS downloads the cleaned masks for bgsb_pool_mask; BGSB_POOL_DETECT keeps them on the device
+ * for bgsb_pool_detect (one more byte per pixel written, no download; the pipeline's kernel stream then waits for the
+ * clean-up and labelling instead of running the next frame set's plugin kernel beside them). 
  * ------------------------------------------------------------------------------------- */
 typedef struct bgsb_pool bgsb_pool;
+enum { BGSB_POOL_MASKS = 1, BGSB_POOL_DETECT = 2 };
 BGSB_API int bgsb_pool_create(bgsb_pool **out, int algo, int nstreams, const int *devices, int ndevices, int w, int h,
                               int ring);
 BGSB_API void bgsb_pool_destroy(bgsb_pool *pool);
-/* As bgsb_pipeline_set_param / bgsb_pipeline_set_morph, applied to every GPU's pipeline; call before the first submit. */
+/* As bgsb_pipeline_set_param / bgsb_pipeline_set_morph, applied to every GPU's pipeline; call before the first submit.
+ * The pool's own key "tableRows" (default 256) sets how many components per stream and frame come back to the host. */
 BGSB_API int bgsb_pool_set_param(bgsb_pool *pool, const char *key, double value);
 BGSB_API int bgsb_pool_set_morph(bgsb_pool *pool, const int *ops, int nops);
 BGSB_API int bgsb_pool_device_of(bgsb_pool *pool, int stream, int *device);
 BGSB_API int bgsb_pool_info(bgsb_pool *pool, int *ngroups, int *ring, int *table_rows);
 BGSB_API uint8_t *bgsb_pool_frame_buffer(bgsb_pool *pool, int stream, int slot);
-BGSB_API int bgsb_pool_submit(bgsb_pool *pool, int slot, int want_masks);
+BGSB_API int bgsb_pool_submit(bgsb_pool *pool, int slot, int flags);
 BGSB_API int bgsb_pool_wait(bgsb_pool *pool, int slot, int *valid);
 BGSB_API const uint8_t *bgsb_pool_mask(bgsb_pool *pool, int stream, int slot);
 BGSB_API int bgsb_pool_components(bgsb_pool *pool, int stream, int slot, bgsb_component *out, int capacity, int *n);
+/* bgsb_pipeline_detect for all N streams of a waited-for slot (arguments indexed by global stream id): the clustering
+ * on the host from the downloaded tables, then per GPU one moments launch over its streams' masks, all GPUs at once.
+ * A stream with more components than "tableRows" gets status[s] = BGSB_ERR_CAPACITY and its detector does not advance;
+ * the others complete, and the call returns BGSB_ERR_CAPACITY.  BGSB_ERR_STATE when the slot was not submitted with
+ * BGSB_POOL_DETECT, has not been waited for, or holds a warm-up frame. */
+BGSB_API int bgsb_pool_detect(bgsb_pool *pool, int slot, bgsb_blobdetector *const *bds, const bgsb_blob *const *old_blobs,
+                              const int *n_old, bgsb_blob *new_blobs, int *result, bgsb_blob *frame_blobs, int *n_frame,
+                              int *status);
 
 /* ---------------------------------------------------------------------------------------
  * Synthetic video of SURVEY 8(d) generated on the device (bench / tests only):

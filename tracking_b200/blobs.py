@@ -108,6 +108,30 @@ class ConnectedComponents:
         return [[int(out[6 * i + j]) for j in range(6)] for i in range(len(rects))]
 
 
+def detect_streams(fn, handle_args, detectors, old_blobs):
+    """bgsb_pipeline_detect / bgsb_pool_detect: per stream (result, new_blob | None, frame_blobs), or None for a stream
+    whose status is not BGSB_OK (its detector did not advance).  old_blobs: None or per stream a list of (x, y, w, h)."""
+    S = len(detectors)
+    bds = (C.c_void_p * S)(*[d._h for d in detectors])
+    old_arrs = [(capi.Blob * max(len(o), 1))(*[capi.Blob(*o_[:4], 0) for o_ in o]) for o in (old_blobs or [()] * S)]
+    olds = (C.POINTER(capi.Blob) * S)(*[C.cast(a, C.POINTER(capi.Blob)) for a in old_arrs])
+    n_old = (C.c_int * S)(*[len(o) for o in (old_blobs or [()] * S)])
+    new, fr = (capi.Blob * S)(), (capi.Blob * (10 * S))()
+    res, n_fr, status = (C.c_int * S)(), (C.c_int * S)(), (C.c_int * S)()
+    rc = fn(*handle_args, bds, olds, n_old, new, res, fr, n_fr, status)
+    if rc not in (capi.OK, capi.ERR_CAPACITY):
+        capi.check(rc)
+    out = []
+    for s, d in enumerate(detectors):
+        if status[s] != capi.OK:
+            out.append(None)
+            continue
+        d.frame_blobs = [(b.x, b.y, b.w, b.h) for b in fr[10 * s:10 * s + n_fr[s]]]
+        nb = (new[s].x, new[s].y, new[s].w, new[s].h) if res[s] else None
+        out.append((res[s], nb, d.frame_blobs))
+    return out
+
+
 class CvBlobDetectorCC:
     """DetectNewBlob(pImg, pFGMask, pNewBlobList, pOldBlobList) -> int."""
 

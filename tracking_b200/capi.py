@@ -19,6 +19,7 @@ ALGO_DP_ADAPTIVE_MEDIAN, ALGO_DP_MEAN, ALGO_DP_WREN_GA = 9, 12, 13     # the DP 
 ALGO_DP_PRATI_MEDIOD = 14
 ALGO_SIGMA_DELTA = 35
 MORPH_ERODE, MORPH_DILATE = 0, 1
+POOL_MASKS, POOL_DETECT = 1, 2
 
 
 class BgsbError(RuntimeError):
@@ -107,6 +108,8 @@ SIGNATURES = {
     "bgsb_pipeline_components": (C.c_int, [vp, C.c_int, C.POINTER(Component), C.c_int, intp]),
     "bgsb_pipeline_tables_dev": (C.c_int, [vp, vp, C.c_int, vp]),
     "bgsb_pipeline_rect_moments": (C.c_int, [vp, C.c_int, i32p, C.c_int, C.POINTER(C.c_uint64)]),
+    "bgsb_pipeline_detect": (C.c_int, [vp, C.POINTER(vp), C.POINTER(C.POINTER(Blob)), intp, C.POINTER(Blob), intp,
+                                       C.POINTER(Blob), intp, intp]),
     "bgsb_pool_create": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, intp, C.c_int, C.c_int, C.c_int, C.c_int]),
     "bgsb_pool_destroy": (None, [vp]),
     "bgsb_pool_set_param": (C.c_int, [vp, C.c_char_p, C.c_double]),
@@ -118,6 +121,8 @@ SIGNATURES = {
     "bgsb_pool_wait": (C.c_int, [vp, C.c_int, intp]),
     "bgsb_pool_mask": (vp, [vp, C.c_int, C.c_int]),
     "bgsb_pool_components": (C.c_int, [vp, C.c_int, C.c_int, C.POINTER(Component), C.c_int, intp]),
+    "bgsb_pool_detect": (C.c_int, [vp, C.c_int, C.POINTER(vp), C.POINTER(C.POINTER(Blob)), intp, C.POINTER(Blob), intp,
+                                   C.POINTER(Blob), intp, intp]),
     "bgsb_synth_frames_dev": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint32, vp]),
     "bgsb_synth_churn_frames_dev": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint32, vp]),
 }

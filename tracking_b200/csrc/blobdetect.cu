@@ -7,6 +7,8 @@
 //   1-2  threshold 128 + external contours         -> bgsb_ccl (GPU)
 //   3    cvSeqPartition of contour rects (CompareContour)      -> partition_rects()
 //   4    union rect per cluster, cvMoments of the mask inside it -> bgsb_ccl_rect_moments (GPU sums)
+// Steps 3 and 5-7 are detect_rects (before the moments) and detect_finish (after them); bgsb_pipeline_detect and
+// bgsb_pool_detect run them around one moments launch for all their streams.
 //   5    drop small blobs and blobs overlapping tracked ones
 //   6    insertion sort by w*h (descending), keep 10
 //   7    track lists over the last `Latency` frames, uniform-motion test, emit best new blob
@@ -17,7 +19,7 @@
 #include <algorithm>
 #include <vector>
 
-#include "common.cuh"
+#include "ccl_internal.h"
 
 using namespace bgsb;
 
@@ -117,47 +119,18 @@ static int ensure_ccl(bgsb_blobdetector *bd, int w, int h)
     return BGSB_OK;
 }
 
-// the part after the mask is on the device
-static int detect_impl(bgsb_blobdetector *bd, const uint8_t *d_mask, int w, int h, const bgsb_blob *old_blobs,
-                       int n_old, bgsb_blob *new_blobs, int new_cap, int *n_new, int *result,
-                       bgsb_blob *frame_blobs, int frame_cap, int *n_frame, cudaStream_t stream)
-{
-    const int SEQ_SIZE = bd->latency;
-    static const bool trace = getenv("BGSB_TRACE_DETECT") != nullptr;     // stage times on stderr (debugging aid)
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    auto us = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-        return std::chrono::duration<double, std::micro>(b - a).count();
-    };
-    const auto t0 = now();
-    int rc = ensure_ccl(bd, w, h);
-    if (rc) return rc;
-    rc = bgsb_ccl_label_dev(bd->ccl, d_mask, w, h, bd->zero_border, nullptr, stream);
-    if (rc) return rc;
-    const auto t1 = now();
-    int ncomp = 0;
-    if (bd->comps.size() < 2048) bd->comps.resize(2048);     // one round trip in the common case
-    rc = bgsb_ccl_components(bd->ccl, bd->comps.data(), (int)bd->comps.size(), &ncomp);
-    if (rc == BGSB_ERR_CAPACITY && ncomp > (int)bd->comps.size()) {
-        bd->comps.resize(ncomp);
-        rc = bgsb_ccl_components(bd->ccl, bd->comps.data(), (int)bd->comps.size(), &ncomp);
-    }
-    if (rc) return rc;
-    const auto t2 = now();
+namespace bgsb {
 
+// (a) component table (raster order) -> the rectangles whose moments step 4 takes
+void detect_rects(const bgsb_blobdetector *bd, const bgsb_component *comps, int ncomp, int w, int h,
+                  std::vector<int32_t> &out)
+{
     // cvFindContours(RETR_EXTERNAL) lists outer contours in REVERSE raster order of their first pixels
     std::vector<Rect> rects;
     for (int i = ncomp - 1; i >= 0; i--) {
-        const bgsb_component &c = bd->comps[i];
+        const bgsb_component &c = comps[i];
         if (c.external) rects.push_back({c.x, c.y, c.w, c.h});
     }
-
-    // ---- shift blob lists (m_pBlobLists) ----
-    if ((int)bd->lists.size() != SEQ_SIZE) bd->lists.assign(SEQ_SIZE, {});
-    for (int i = SEQ_SIZE - 1; i > 0; --i) bd->lists[i] = std::move(bd->lists[i - 1]);
-    bd->lists[0].clear();
-
-    // ---- create blobs ----
-    std::vector<bgsb_blob> blobs;
     std::vector<Rect> qrects;
     if (bd->Clastering) {                       // cvFindBlobsByCCClasters
         std::vector<int> cls;
@@ -179,21 +152,24 @@ static int detect_impl(bgsb_blobdetector *bd, const uint8_t *d_mask, int w, int 
             qrects.push_back(r);
         }
     }
-    const auto t3 = now();
-    std::vector<uint64_t> mom(qrects.size() * 6 + 6);
-    if (!qrects.empty()) {
-        std::vector<int32_t> flat(qrects.size() * 4);
-        for (size_t i = 0; i < qrects.size(); i++) {
-            flat[4 * i] = qrects[i].x; flat[4 * i + 1] = qrects[i].y; flat[4 * i + 2] = qrects[i].w; flat[4 * i + 3] = qrects[i].h;
-        }
-        rc = bgsb_ccl_rect_moments(bd->ccl, flat.data(), (int)qrects.size(), mom.data());
-        if (rc) return rc;
-    }
-    if (trace)
-        fprintf(stderr, "detect: launch %.0f us, components(%d) %.0f us, clustering(%zu rects) %.0f us, moments(%zu) %.0f us\n",
-                us(t0, t1), ncomp, us(t1, t2), rects.size(), us(t2, t3), qrects.size(), us(t3, now()));
-    for (size_t i = 0; i < qrects.size(); i++) {
-        const Rect &R = qrects[i];
+    for (const Rect &R : qrects) out.insert(out.end(), {R.x, R.y, R.w, R.h});
+}
+
+// (b) the rectangles and their moments + the tracked blobs -> blob list, filters, top-10, tracks, result
+void detect_finish(bgsb_blobdetector *bd, const int32_t *qrects, int nq, const uint64_t *mom, int w, int h,
+                   const bgsb_blob *old_blobs, int n_old, bgsb_blob *new_blobs, int new_cap, int *n_new, int *result,
+                   bgsb_blob *frame_blobs, int frame_cap, int *n_frame)
+{
+    const int SEQ_SIZE = bd->latency;
+    // ---- shift blob lists (m_pBlobLists) ----
+    if ((int)bd->lists.size() != SEQ_SIZE) bd->lists.assign(SEQ_SIZE, {});
+    for (int i = SEQ_SIZE - 1; i > 0; --i) bd->lists[i] = std::move(bd->lists[i - 1]);
+    bd->lists[0].clear();
+
+    // ---- create blobs ----
+    std::vector<bgsb_blob> blobs;
+    for (int i = 0; i < nq; i++) {
+        const Rect R = {qrects[4 * i], qrects[4 * i + 1], qrects[4 * i + 2], qrects[4 * i + 3]};
         double X, Y, XX, YY;
         if (R.h < 1 || R.w < 1) { X = Y = XX = YY = 0; }
         else {
@@ -330,6 +306,66 @@ static int detect_impl(bgsb_blobdetector *bd, const uint8_t *d_mask, int w, int 
         bd->tracks.pop_back();
     }
     if (result) *result = res;
+}
+
+int detect_check(bgsb_blobdetector *const *bds, int S, const bgsb_blob *const *old_blobs, const int *n_old,
+                 int zero_border)
+{
+    BGSB_REQUIRE(bds, "null detectors");
+    BGSB_REQUIRE(!old_blobs || n_old, "old_blobs without n_old");
+    std::vector<const bgsb_blobdetector *> seen(bds, bds + S);
+    std::sort(seen.begin(), seen.end());
+    BGSB_REQUIRE(seen.empty() || seen[0], "a detector is NULL");
+    BGSB_REQUIRE(std::adjacent_find(seen.begin(), seen.end()) == seen.end(), "one detector given for two streams");
+    for (int s = 0; s < S; s++) {
+        // the masks were labelled with the pipeline's setting; a detector's own would label other components
+        BGSB_REQUIRE(bds[s]->zero_border == zero_border, "a detector's zeroBorder differs from the pipeline's");
+        if (old_blobs) BGSB_REQUIRE(n_old[s] >= 0 && (n_old[s] == 0 || old_blobs[s]), "old blob list of a stream");
+    }
+    return BGSB_OK;
+}
+
+}  // namespace bgsb
+
+// label -> (a) -> moments -> (b)
+static int detect_impl(bgsb_blobdetector *bd, const uint8_t *d_mask, int w, int h, const bgsb_blob *old_blobs,
+                       int n_old, bgsb_blob *new_blobs, int new_cap, int *n_new, int *result,
+                       bgsb_blob *frame_blobs, int frame_cap, int *n_frame, cudaStream_t stream)
+{
+    static const bool trace = getenv("BGSB_TRACE_DETECT") != nullptr;     // stage times on stderr (debugging aid)
+    auto now = [] { return std::chrono::steady_clock::now(); };
+    auto us = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
+        return std::chrono::duration<double, std::micro>(b - a).count();
+    };
+    const auto t0 = now();
+    int rc = ensure_ccl(bd, w, h);
+    if (rc) return rc;
+    rc = bgsb_ccl_label_dev(bd->ccl, d_mask, w, h, bd->zero_border, nullptr, stream);
+    if (rc) return rc;
+    const auto t1 = now();
+    int ncomp = 0;
+    if (bd->comps.size() < 2048) bd->comps.resize(2048);     // one round trip in the common case
+    rc = bgsb_ccl_components(bd->ccl, bd->comps.data(), (int)bd->comps.size(), &ncomp);
+    if (rc == BGSB_ERR_CAPACITY && ncomp > (int)bd->comps.size()) {
+        bd->comps.resize(ncomp);
+        rc = bgsb_ccl_components(bd->ccl, bd->comps.data(), (int)bd->comps.size(), &ncomp);
+    }
+    if (rc) return rc;
+    const auto t2 = now();
+    std::vector<int32_t> qrects;
+    detect_rects(bd, bd->comps.data(), ncomp, w, h, qrects);
+    const int nq = (int)qrects.size() / 4;
+    const auto t3 = now();
+    std::vector<uint64_t> mom(6 * (size_t)nq + 6);
+    if (nq) {
+        rc = bgsb_ccl_rect_moments(bd->ccl, qrects.data(), nq, mom.data());
+        if (rc) return rc;
+    }
+    if (trace)
+        fprintf(stderr, "detect: launch %.0f us, components(%d) %.0f us, clustering(%d rects) %.0f us, moments %.0f us\n",
+                us(t0, t1), ncomp, us(t1, t2), nq, us(t2, t3), us(t3, now()));
+    detect_finish(bd, qrects.data(), nq, mom.data(), w, h, old_blobs, n_old, new_blobs, new_cap, n_new, result, frame_blobs,
+                  frame_cap, n_frame);
     return BGSB_OK;
 }
 

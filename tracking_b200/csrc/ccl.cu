@@ -688,29 +688,24 @@ ccl_background_phase_kernel(const __grid_constant__ CclArgs A)
     }
 }
 
-// cvMoments(ROI, binary=0): pixel-value weighted raw moments, ROI-relative coordinates.
-__global__ void __launch_bounds__(256)
-rect_moments_kernel(const uint8_t *__restrict__ mask, int w, int h, const int *__restrict__ rects,
-                    unsigned long long *out)
+// cvMoments(ROI, binary=0): pixel-value weighted raw moments, ROI-relative coordinates, for a batch of
+// (image, rect) records in one launch.  One CTA per tile: rows_per_tile rows of one record, about the same number of
+// pixels whatever the record's width (moment_tiles), so the grid follows the records' area, not their count.  Each warp
+// takes every 8th row of its tile; a row's sums are exact in 32 bits inside each 16-byte load and are widened to
+// 64 bits per load, then folded into the six moments per row.  Rects crossing the image edge are clipped; the
+// coordinates stay relative to the unclipped rect.
+__device__ __forceinline__ int moment_record(const MomRec *__restrict__ recs, int nrec)
 {
-    pdl_entry();
-    const int ri = blockIdx.x;
-    const int rx = rects[4 * ri], ry = rects[4 * ri + 1], rw = rects[4 * ri + 2], rh = rects[4 * ri + 3];
-    unsigned long long m[6] = {0, 0, 0, 0, 0, 0};
-    // each y-slice of blocks takes every gridDim.y-th row
-    for (int yy = blockIdx.y; yy < rh; yy += gridDim.y) {
-        int y = ry + yy;
-        if (y < 0 || y >= h) continue;
-        const uint8_t *row = mask + (size_t)y * w;
-        unsigned long long r0 = 0, r1 = 0, r2 = 0;       // sum v, sum v*x, sum v*x*x over this row
-        for (int xx = threadIdx.x; xx < rw; xx += blockDim.x) {
-            int x = rx + xx;
-            if (x < 0 || x >= w) continue;
-            unsigned long long v = row[x];
-            r0 += v; r1 += v * xx; r2 += v * (unsigned long long)xx * xx;
-        }
-        m[0] += r0; m[1] += r1; m[2] += r0 * yy; m[3] += r2; m[4] += r0 * (unsigned long long)yy * yy; m[5] += r1 * yy;
+    int lo = 0, hi = nrec - 1;                  // the last record whose first tile is <= this CTA's (it has tiles)
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (recs[mid].first_tile <= (int)blockIdx.x) lo = mid; else hi = mid - 1;
     }
+    return lo;
+}
+
+__device__ __forceinline__ void moments_flush(unsigned long long (&m)[6], unsigned long long *out)
+{
     __shared__ unsigned long long red[6][8];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 #pragma unroll
@@ -723,53 +718,161 @@ rect_moments_kernel(const uint8_t *__restrict__ mask, int w, int h, const int *_
     if (threadIdx.x < 6) {
         unsigned long long v = 0;
         for (int i = 0; i < 8; i++) v += red[threadIdx.x][i];
-        if (v) atomicAdd(out + 6 * ri + threadIdx.x, v);
+        if (v) atomicAdd(out + threadIdx.x, v);
     }
 }
 
-// The same sums from a bit-packed {0,255} mask (the pipeline keeps no byte mask): every set bit weighs 255.
+// r0 r1 r2 of one row (sum v, v*x, v*x*x) -> the six moments, yy = the row's ROI-relative y
+__device__ __forceinline__ void moments_add_row(unsigned long long (&m)[6], unsigned long long r0, unsigned long long r1,
+                                                unsigned long long r2, unsigned long long yy)
+{
+    m[0] += r0; m[1] += r1; m[2] += r0 * yy; m[3] += r2; m[4] += r0 * yy * yy; m[5] += r1 * yy;
+}
+
+// The clipped tile of this CTA: rows [y0, y1) and columns [xa, xb) of the image, rx / ry the rect's origin.
+struct MomTile { int img, rx, ry, xa, xb, y0, y1; };
+
+__device__ __forceinline__ MomTile moment_tile(const MomRec &R, int w, int h)
+{
+    MomTile t;
+    t.img = R.image; t.rx = R.x; t.ry = R.y;
+    t.xa = max(R.x, 0); t.xb = min(R.x + R.w, w);
+    const int ya = max(R.y, 0), yb = min(R.y + R.h, h);
+    t.y0 = ya + ((int)blockIdx.x - R.first_tile) * R.rows_per_tile;
+    t.y1 = min(yb, t.y0 + R.rows_per_tile);
+    return t;
+}
+
+// byte masks [images][h][w]
 __global__ void __launch_bounds__(256)
-rect_moments_bits_kernel(const unsigned *__restrict__ bits, int w, int h, int wpr, const int *__restrict__ rects,
-                         unsigned long long *out)
+rect_moments_kernel(const uint8_t *__restrict__ mask, int w, int h, const MomRec *__restrict__ recs, int nrec,
+                    unsigned long long *out)
 {
     pdl_entry();
-    const int ri = blockIdx.x;
-    const int rx = rects[4 * ri], ry = rects[4 * ri + 1], rw = rects[4 * ri + 2], rh = rects[4 * ri + 3];
-    const int xa = max(rx, 0), xb = min(rx + rw, w);             // [xa, xb) inside the image
+    const int ri = moment_record(recs, nrec);
+    const MomTile t = moment_tile(recs[ri], w, h);
+    const int lane = threadIdx.x & 31;
     unsigned long long m[6] = {0, 0, 0, 0, 0, 0};
-    if (xa < xb) {
-        const int k0 = xa >> 5, k1 = (xb - 1) >> 5;
-        for (int yy = blockIdx.y; yy < rh; yy += gridDim.y) {
-            const int y = ry + yy;
-            if (y < 0 || y >= h) continue;
-            unsigned long long r0 = 0, r1 = 0, r2 = 0;
-            for (int k = k0 + (int)threadIdx.x; k <= k1; k += blockDim.x) {
-                unsigned v = bits[(size_t)y * wpr + k];
-                if (k == k0) v &= 0xffffffffu << (xa & 31);
-                if (k == k1 && (xb & 31)) v &= 0xffffffffu >> (32 - (xb & 31));
-                while (v) {
-                    const int b = __ffs(v) - 1; v &= v - 1;
-                    const unsigned long long xx = (unsigned long long)(k * 32 + b - rx);
-                    r0 += 255ull; r1 += 255ull * xx; r2 += 255ull * xx * xx;
-                }
-            }
-            m[0] += r0; m[1] += r1; m[2] += r0 * yy; m[3] += r2; m[4] += r0 * (unsigned long long)yy * yy; m[5] += r1 * yy;
+    for (int y = t.y0 + (int)(threadIdx.x >> 5); y < t.y1; y += 8) {
+        const uint8_t *row = mask + ((size_t)t.img * h + y) * w;
+        const uintptr_t p0 = (uintptr_t)(row + t.xa), p1 = (uintptr_t)(row + t.xb);
+        // [p0, a) head and [b, p1) tail bytes (< 16 each) one per lane, [a, b) in aligned 16-byte loads
+        const uintptr_t a = min((p0 + 15) & ~(uintptr_t)15, p1), b = max(p1 & ~(uintptr_t)15, a);
+        unsigned long long r0 = 0, r1 = 0, r2 = 0;
+        const uintptr_t q = lane < 16 ? p0 + lane : b + (lane - 16);
+        if (q < (lane < 16 ? a : p1)) {
+            const unsigned long long v = *(const uint8_t *)q, xx = (unsigned long long)((const uint8_t *)q - row - t.rx);
+            r0 = v; r1 = v * xx; r2 = v * xx * xx;
         }
+        for (uintptr_t c = a + 16 * (uintptr_t)lane; c < b; c += 512) {
+            const uint4 v = *(const uint4 *)c;
+            if ((v.x | v.y | v.z | v.w) == 0) continue;
+            // byte k of the load weighs 1, k and k*k (IDP.4A: four byte products per instruction)
+            const unsigned s0 = __dp4a(v.x, 0x01010101u, __dp4a(v.y, 0x01010101u, __dp4a(v.z, 0x01010101u, __dp4a(v.w, 0x01010101u, 0u))));
+            const unsigned s1 = __dp4a(v.x, 0x03020100u, __dp4a(v.y, 0x07060504u, __dp4a(v.z, 0x0b0a0908u, __dp4a(v.w, 0x0f0e0d0cu, 0u))));
+            const unsigned s2 = __dp4a(v.x, 0x09040100u, __dp4a(v.y, 0x31241910u, __dp4a(v.z, 0x79645140u, __dp4a(v.w, 0xe1c4a990u, 0u))));
+            const unsigned long long x0 = (unsigned long long)((const uint8_t *)c - row - t.rx);
+            r0 += s0; r1 += s1 + x0 * s0; r2 += s2 + 2 * x0 * s1 + x0 * x0 * s0;
+        }
+        moments_add_row(m, r0, r1, r2, (unsigned long long)(y - t.ry));
     }
-    __shared__ unsigned long long red[6][8];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    moments_flush(m, out + 6 * ri);
+}
+
+// The same sums from bit-packed {0,255} masks [images][h][wpr] (the pipeline keeps no byte mask): every set bit weighs
+// 255.  A word's sums of x and x*x over its set bits come from popcounts of the bit-position masks.
+__device__ __forceinline__ unsigned bitpos_mask(int j)
+{
+    return j == 0 ? 0xaaaaaaaau : j == 1 ? 0xccccccccu : j == 2 ? 0xf0f0f0f0u : j == 3 ? 0xff00ff00u : 0xffff0000u;
+}
+
+__global__ void __launch_bounds__(256)
+rect_moments_bits_kernel(const unsigned *__restrict__ bits, int w, int h, int wpr, const MomRec *__restrict__ recs,
+                         int nrec, unsigned long long *out)
+{
+    pdl_entry();
+    const int ri = moment_record(recs, nrec);
+    const MomTile t = moment_tile(recs[ri], w, h);
+    const int lane = threadIdx.x & 31;
+    unsigned long long m[6] = {0, 0, 0, 0, 0, 0};
+    const int k0 = t.xa >> 5, k1 = (t.xb - 1) >> 5;
+    for (int y = t.y0 + (int)(threadIdx.x >> 5); y < t.y1; y += 8) {
+        const unsigned *row = bits + ((size_t)t.img * h + y) * wpr;
+        unsigned long long r0 = 0, r1 = 0, r2 = 0;
+        for (int k = k0 + lane; k <= k1; k += 32) {
+            unsigned v = row[k];
+            if (k == k0) v &= 0xffffffffu << (t.xa & 31);
+            if (k == k1 && (t.xb & 31)) v &= 0xffffffffu >> (32 - (t.xb & 31));
+            if (!v) continue;
+            unsigned s0 = __popc(v), s1 = 0, s2 = 0;          // sum 1, b, b*b over the set bits b
 #pragma unroll
-    for (int i = 0; i < 6; i++) {
-        unsigned long long v = m[i];
-        for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
-        if (lane == 0) red[i][wid] = v;
+            for (int j = 0; j < 5; j++) {
+                const unsigned vj = v & bitpos_mask(j);
+                s1 += __popc(vj) << j;
+                s2 += __popc(vj) << (2 * j);
+#pragma unroll
+                for (int i = j + 1; i < 5; i++) s2 += __popc(vj & bitpos_mask(i)) << (i + j + 1);
+            }
+            // x = 32k + b - rx; the word's base may lie left of the rect (its bits there are masked off), and the
+            // modular 64-bit products cancel exactly
+            const unsigned long long x0 = (unsigned long long)(long long)(32 * k - t.rx);
+            r0 += s0; r1 += s1 + x0 * s0; r2 += s2 + 2 * x0 * s1 + x0 * x0 * s0;
+        }
+        moments_add_row(m, 255ull * r0, 255ull * r1, 255ull * r2, (unsigned long long)(y - t.ry));
     }
-    __syncthreads();
-    if (threadIdx.x < 6) {
-        unsigned long long v = 0;
-        for (int i = 0; i < 8; i++) v += red[threadIdx.x][i];
-        if (v) atomicAdd(out + 6 * ri + threadIdx.x, v);
+    moments_flush(m, out + 6 * ri);
+}
+
+int moment_tiles(MomRec *recs, int n, int w, int h)
+{
+    long long tiles = 0;
+    for (int i = 0; i < n; i++) {
+        MomRec &R = recs[i];
+        const long long cols = std::min<long long>((long long)R.x + R.w, w) - std::max(R.x, 0);
+        const long long rows = std::min<long long>((long long)R.y + R.h, h) - std::max(R.y, 0);
+        // a row costs its pixels plus a fixed overhead of ~256 pixels' worth; a tile is ~16K pixels' worth, whole warps
+        R.rows_per_tile = 8 * (int)std::max<long long>(1, (16384 / (std::max<long long>(cols, 0) + 256) + 7) / 8);
+        R.first_tile = (int)tiles;
+        if (cols > 0 && rows > 0) tiles += (rows + R.rows_per_tile - 1) / R.rows_per_tile;
     }
+    return (int)tiles;
+}
+
+int MomentBatch::reserve(int n)
+{
+    if (n <= cap) return BGSB_OK;
+    release();
+    const int c = std::max(1024, 2 * n);
+    BGSB_CUDA(cudaMallocHost(&h_rec, (size_t)c * sizeof(MomRec)));
+    BGSB_CUDA(cudaMallocHost(&h_mom, (size_t)c * 48));
+    BGSB_CUDA(cudaMalloc(&d_rec, (size_t)c * sizeof(MomRec)));
+    BGSB_CUDA(cudaMalloc(&d_mom, (size_t)c * 48));
+    cap = c;
+    return BGSB_OK;
+}
+
+void MomentBatch::release()
+{
+    if (h_rec) cudaFreeHost(h_rec);
+    if (h_mom) cudaFreeHost(h_mom);
+    cudaFree(d_rec); cudaFree(d_mom);
+    h_rec = nullptr; h_mom = nullptr; d_rec = nullptr; d_mom = nullptr; cap = 0;
+}
+
+int MomentBatch::enqueue(const uint8_t *mask, const unsigned *bits, int w, int h, int n, cudaStream_t st)
+{
+    if (n == 0) return BGSB_OK;
+    const int ntiles = moment_tiles(h_rec, n, w, h);
+    BGSB_CUDA(cudaMemcpyAsync(d_rec, h_rec, (size_t)n * sizeof(MomRec), cudaMemcpyHostToDevice, st));
+    BGSB_CUDA(cudaMemsetAsync(d_mom, 0, (size_t)n * 48, st));
+    if (ntiles > 0) {
+        if (mask) launch_pdl(rect_moments_kernel, dim3(ntiles), dim3(256), 0, st, mask, w, h, (const MomRec *)d_rec, n, d_mom);
+        else launch_pdl(rect_moments_bits_kernel, dim3(ntiles), dim3(256), 0, st, bits, w, h, (w + 31) / 32,
+                        (const MomRec *)d_rec, n, d_mom);
+        BGSB_LAUNCH_CHECK();
+    }
+    BGSB_CUDA(cudaMemcpyAsync(h_mom, d_mom, (size_t)n * 48, cudaMemcpyDeviceToHost, st));
+    return BGSB_OK;
 }
 
 // The component tables of all images of the last call, decoded, in one dense buffer: per image 8 ints of header
@@ -966,7 +1069,7 @@ void bgsb_ccl_destroy(bgsb_ccl *c)
     cudaFree(c->d_bits); cudaFree(c->d_parent);
     cudaFree(c->d_outer); cudaFree(c->d_mask_own); cudaFree(c->d_comp); cudaFree(c->d_ncomp);
     cudaFree(c->d_chunkcount); cudaFree(c->d_chunkprefix); cudaFree(c->d_done); cudaFree(c->d_need_bg); cudaFree(c->d_labels_own);
-    cudaFree(c->d_rects); cudaFree(c->d_mom);
+    c->moments.release();
     if (c->h_pin) cudaFreeHost(c->h_pin);
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
     delete c;
@@ -1050,35 +1153,18 @@ int bgsb_ccl_rect_moments_of(bgsb_ccl *c, int image, const int32_t *rects, int n
     BGSB_REQUIRE(c && out && (rects || nrects == 0), "null");
     if (!c->labelled) { set_error("bgsb_ccl_rect_moments: nothing labelled yet"); return BGSB_ERR_STATE; }
     BGSB_REQUIRE(image >= 0 && image < c->nimages, "image index");
+    BGSB_REQUIRE(nrects >= 0, "nrects >= 0");
     if (nrects == 0) return BGSB_OK;
     BGSB_CUDA(cudaSetDevice(c->device));
-    cudaStream_t st = c->last_stream;
-    if (nrects > c->rect_cap) {                              // grows rarely; no allocator calls on the per-frame path
-        cudaFree(c->d_rects); cudaFree(c->d_mom); c->d_rects = nullptr; c->d_mom = nullptr; c->rect_cap = 0;
-        const int cap = std::max(1024, nrects * 2);
-        BGSB_CUDA(cudaMalloc(&c->d_rects, (size_t)cap * 16));
-        BGSB_CUDA(cudaMalloc(&c->d_mom, (size_t)cap * 48));
-        c->rect_cap = cap;
-    }
-    if (!c->h_pin) BGSB_CUDA(cudaMallocHost(&c->h_pin, 64 + (size_t)bgsb_ccl::PIN_COMPS * sizeof(CompRaw)));
-    const size_t pin_bytes = (size_t)bgsb_ccl::PIN_COMPS * sizeof(CompRaw);
-    const bool staged = (size_t)nrects * 48 <= pin_bytes;     // moments come back through pinned memory when they fit
-    BGSB_CUDA(cudaMemcpyAsync(c->d_rects, rects, (size_t)nrects * 16, cudaMemcpyHostToDevice, st));
-    BGSB_CUDA(cudaMemsetAsync(c->d_mom, 0, (size_t)nrects * 48, st));
-    dim3 grid(nrects, 16);
-    if (c->last_mask)
-        launch_pdl(rect_moments_kernel, dim3(grid), dim3(256), 0, st, c->last_mask + (size_t)image * c->w * c->h, c->w, c->h,
-                   c->d_rects, c->d_mom);
-    else {
-        const int wpr = (c->w + 31) / 32;
-        launch_pdl(rect_moments_bits_kernel, dim3(grid), dim3(256), 0, st, c->last_bits + (size_t)image * wpr * c->h, c->w, c->h,
-                   wpr, c->d_rects, c->d_mom);
-    }
-    BGSB_LAUNCH_CHECK();
-    BGSB_CUDA(cudaMemcpyAsync(staged ? (void *)(c->h_pin + 64) : (void *)out, c->d_mom, (size_t)nrects * 48,
-                              cudaMemcpyDeviceToHost, st));
-    BGSB_CUDA(cudaStreamSynchronize(st));
-    if (staged) memcpy(out, c->h_pin + 64, (size_t)nrects * 48);
+    // a batch whose records all name this image (buffers grow rarely: no allocator calls on the per-frame path)
+    int rc = c->moments.reserve(nrects);
+    if (rc) return rc;
+    for (int i = 0; i < nrects; i++)
+        c->moments.h_rec[i] = MomRec{image, rects[4 * i], rects[4 * i + 1], rects[4 * i + 2], rects[4 * i + 3], 0, 0, 0};
+    rc = c->moments.enqueue(c->last_mask, c->last_bits, c->w, c->h, nrects, c->last_stream);
+    if (rc) return rc;
+    BGSB_CUDA(cudaStreamSynchronize(c->last_stream));
+    memcpy(out, c->moments.h_mom, (size_t)nrects * 48);
     return BGSB_OK;
 }
 

@@ -1,9 +1,46 @@
 // Internal interface of the labeller (ccl.cu) for the other translation units of the library (pipeline.cu).
 #pragma once
+#include <vector>
+
 #include "common.cuh"
 
 namespace bgsb {
 struct CompRaw { int label, first_index, xmin, ymin, xmax, ymax, area, external; };
+
+// One rectangle of a batched cvMoments query: the image it lies in and its x, y, w, h (may cross the image edge), plus
+// the tiling moment_tiles() fills in.
+struct MomRec { int image, x, y, w, h, rows_per_tile, first_tile, pad; };
+
+// Split the records' clipped rows into tiles of about equal work (one CTA each); -> the number of tiles.
+int moment_tiles(MomRec *recs, int n, int w, int h);
+
+// Host and device staging of a batched moments query, grown on demand (no allocator calls once large enough).
+struct MomentBatch {
+    MomRec *h_rec = nullptr, *d_rec = nullptr;          // pinned / device records
+    unsigned long long *h_mom = nullptr, *d_mom = nullptr;   // pinned / device sums, 6 per record
+    int cap = 0;
+    int reserve(int n);
+    void release();
+    // h_rec[0, n) up, one moments launch over images of w x h -- byte masks [images][h][w] when mask != NULL, else
+    // bit-packed {0,255} masks [images][h][wpr] -- and h_mom[0, 6n) down: m00 m10 m01 m20 m02 m11 per record
+    // (ROI-relative, exact).  Asynchronous on `stream`.
+    int enqueue(const uint8_t *mask, const unsigned *bits, int w, int h, int n, cudaStream_t stream);
+};
+
+// CvBlobDetectorCC::DetectNewBlob (blobdetect.cu) in two halves around the moments of step 4:
+//   detect_rects : component table (raster order, every component) -> the rectangles step 4 weighs (external ones in
+//                  reverse raster order, clustered and united), appended to `rects` as x, y, w, h
+//   detect_finish: those rectangles with their moments (6 per rectangle) and the tracked blobs -> blob list, filters,
+//                  top-10, track update and result; advances the detector
+void detect_rects(const bgsb_blobdetector *bd, const bgsb_component *comps, int ncomp, int w, int h,
+                  std::vector<int32_t> &rects);
+void detect_finish(bgsb_blobdetector *bd, const int32_t *rects, int nrects, const uint64_t *mom, int w, int h,
+                   const bgsb_blob *old_blobs, int n_old, bgsb_blob *new_blobs, int new_cap, int *n_new, int *result,
+                   bgsb_blob *frame_blobs, int frame_cap, int *n_frame);
+// The arguments of the batched entry points: S distinct non-NULL detectors whose "zeroBorder" equals the one the masks
+// were labelled with, and per-stream old blob lists (old_blobs may be NULL: no tracked blobs).
+int detect_check(bgsb_blobdetector *const *bds, int S, const bgsb_blob *const *old_blobs, const int *n_old,
+                 int zero_border);
 }
 
 struct bgsb_ccl {
@@ -32,13 +69,11 @@ struct bgsb_ccl {
     cudaStream_t last_stream = nullptr;
     cudaStream_t own_stream = nullptr;
     bool labelled = false;
-    // host round trips of the per-frame path: pinned staging (count + the first PIN_COMPS table rows, or moments) and
-    // device buffers for the rectangle queries that live as long as the context (no allocator calls per frame)
+    // host round trips of the per-frame path: pinned staging (count + the first PIN_COMPS table rows) and the
+    // rectangle queries' buffers, which live as long as the context (no allocator calls per frame)
     static constexpr int PIN_COMPS = 2048;
     uint8_t *h_pin = nullptr;               // 64 + PIN_COMPS * sizeof(CompRaw) bytes
-    int *d_rects = nullptr;
-    unsigned long long *d_mom = nullptr;
-    int rect_cap = 0;
+    bgsb::MomentBatch moments;
 };
 
 namespace bgsb {

@@ -42,6 +42,12 @@ struct bgsb_pipeline {
     uint8_t *d_fg[NSLOT] = {};                          // [S][h][w] byte masks of plugins that cannot emit bits
     bool labelled = false;
     bool raw_chain = false;                             // the last labelled frame: threshold off, chain on (no moments)
+    bool last_valid = false;                            // the last process call produced (and labelled) a mask
+    int label_zero_border = 1;                          // the "zeroBorder" the last frame was labelled with
+    // bgsb_pipeline_detect: gathered tables (DETECT_ROWS per stream) and the batched moments query
+    static constexpr int DETECT_ROWS = 256;
+    int32_t *d_tab = nullptr, *h_tab = nullptr;
+    bgsb::MomentBatch moments;
     // Clean-up + labelling of frame t run on the pipeline's own high-priority stream, so that they overlap the plugin
     // kernel of frame t+1 (their launches are latency-bound and leave the SMs almost empty): the caller's stream only
     // waits for them when it has to (device outputs requested, or bgsb_pipeline_join_dev).
@@ -56,6 +62,10 @@ static void pipeline_free(bgsb_pipeline *p)
 {
     for (int i = 0; i < bgsb_pipeline::NSLOT; i++) { cudaFree(p->d_raw[i]); cudaFree(p->d_fg[i]); p->d_raw[i] = nullptr; p->d_fg[i] = nullptr; p->chain_used[i] = false; }
     cudaFree(p->d_clean); p->d_clean = nullptr;
+    cudaFree(p->d_tab); p->d_tab = nullptr;
+    if (p->h_tab) cudaFreeHost(p->h_tab);
+    p->h_tab = nullptr;
+    p->moments.release();
     p->last_slot = -1;
     if (p->ccl) { bgsb_ccl_destroy(p->ccl); p->ccl = nullptr; }
     p->w = p->h = 0; p->labelled = false;
@@ -157,6 +167,7 @@ int bgsb_pipeline_process_dev(bgsb_pipeline *p, const uint8_t *d_frames, int w, 
     BGSB_CUDA(cudaSetDevice(p->device));
     cudaStream_t stream = (cudaStream_t)stream_;
     if (valid) *valid = 0;
+    p->last_valid = false;
     nvtxRangePushA("bgsb_pipeline: plugin + clean-up + labelling");
     struct NvtxPop { ~NvtxPop() { nvtxRangePop(); } } nvtx_pop;
     int rc = pipeline_geometry(p, w, h);
@@ -244,6 +255,8 @@ int bgsb_pipeline_process_dev(bgsb_pipeline *p, const uint8_t *d_frames, int w, 
     if (d_mask || d_labels) BGSB_CUDA(cudaStreamWaitEvent(stream, p->ev_chain[slot], 0));
     p->labelled = true;
     p->raw_chain = raw_chain;
+    p->last_valid = true;
+    p->label_zero_border = p->zero_border;
     if (valid) *valid = 1;
     return BGSB_OK;
 }
@@ -285,6 +298,70 @@ int bgsb_pipeline_rect_moments(bgsb_pipeline *p, int stream_index, const int32_t
         return BGSB_ERR_ARG;
     }
     return bgsb_ccl_rect_moments_of(p->ccl, stream_index, rects, nrects, out);
+}
+
+int bgsb_pipeline_detect(bgsb_pipeline *p, bgsb_blobdetector *const *bds, const bgsb_blob *const *old_blobs,
+                         const int *n_old, bgsb_blob *new_blobs, int *result, bgsb_blob *frame_blobs, int *n_frame,
+                         int *status)
+{
+    BGSB_REQUIRE(p && new_blobs && result && status, "null");
+    if (!p->last_valid) { set_error("bgsb_pipeline_detect: the last frame produced no mask (plugin warm-up)"); return BGSB_ERR_STATE; }
+    if (p->raw_chain) {
+        set_error("bgsb_pipeline_detect: with enableThreshold = 0 and an erode / dilate chain the reference weighs the "
+                  "grey-level cleaned mask, which the pipeline does not compute");
+        return BGSB_ERR_ARG;
+    }
+    int rc = detect_check(bds, p->nstreams, old_blobs, n_old, p->label_zero_border);
+    if (rc) return rc;
+    BGSB_CUDA(cudaSetDevice(p->device));
+    const int S = p->nstreams, R = bgsb_pipeline::DETECT_ROWS, w = p->w, h = p->h;
+    const size_t tab_ints = (size_t)(R + 1) * 8;
+    if (!p->d_tab) {
+        BGSB_CUDA(cudaMalloc(&p->d_tab, S * tab_ints * sizeof(int32_t)));
+        BGSB_CUDA(cudaMallocHost(&p->h_tab, S * tab_ints * sizeof(int32_t)));
+    }
+    // every stream's table in one gather and one download, behind the labelling on the pipeline's stream
+    rc = ccl_gather_tables(p->ccl, p->d_tab, R, p->side);
+    if (rc) return rc;
+    BGSB_CUDA(cudaMemcpyAsync(p->h_tab, p->d_tab, S * tab_ints * sizeof(int32_t), cudaMemcpyDeviceToHost, p->side));
+    BGSB_CUDA(cudaStreamSynchronize(p->side));
+    // (a) per stream; a stream with more components than the gathered rows fetches its whole table
+    std::vector<int32_t> rects;
+    std::vector<int> first(S + 1, 0);
+    std::vector<bgsb_component> big;
+    for (int s = 0; s < S; s++) {
+        const int32_t *t = p->h_tab + s * tab_ints;
+        int n = t[0];
+        const bgsb_component *comps = reinterpret_cast<const bgsb_component *>(t + 8);
+        if (n > R) {
+            big.resize(n);
+            rc = bgsb_ccl_components_of(p->ccl, s, big.data(), n, &n);
+            if (rc) return rc;
+            comps = big.data();
+        }
+        detect_rects(bds[s], comps, n, w, h, rects);
+        first[s + 1] = (int)rects.size() / 4;
+    }
+    // one moments launch for all streams, on the source the labeller weighed
+    const int nrec = first[S];
+    rc = p->moments.reserve(nrec);
+    if (rc) return rc;
+    for (int s = 0; s < S; s++)
+        for (int i = first[s]; i < first[s + 1]; i++)
+            p->moments.h_rec[i] = MomRec{s, rects[4 * i], rects[4 * i + 1], rects[4 * i + 2], rects[4 * i + 3], 0, 0, 0};
+    rc = p->moments.enqueue(p->ccl->last_mask, p->ccl->last_bits, w, h, nrec, p->side);
+    if (rc) return rc;
+    BGSB_CUDA(cudaStreamSynchronize(p->side));
+    // (b) per stream
+    for (int s = 0; s < S; s++) {
+        int n_new = 0;
+        detect_finish(bds[s], rects.data() + 4 * first[s], first[s + 1] - first[s],
+                      reinterpret_cast<const uint64_t *>(p->moments.h_mom) + 6 * first[s], w, h,
+                      old_blobs ? old_blobs[s] : nullptr, old_blobs ? n_old[s] : 0, new_blobs + s, 1, &n_new, result + s,
+                      frame_blobs ? frame_blobs + 10 * s : nullptr, 10, n_frame ? n_frame + s : nullptr);
+        status[s] = BGSB_OK;
+    }
+    return BGSB_OK;
 }
 
 }  // extern "C"

@@ -22,7 +22,7 @@
 #include <thread>
 #include <vector>
 
-#include "common.cuh"
+#include "ccl_internal.h"
 #include "kernels.h"
 
 using namespace bgsb;
@@ -31,7 +31,8 @@ namespace {
 
 constexpr int POOL_RING_MAX = 8;
 
-struct Job { int slot; int want_masks; uint64_t seq; };
+// flags: BGSB_POOL_MASKS / BGSB_POOL_DETECT of bgsb_pool_submit; a DETECT job is the moments query of bgsb_pool_detect
+struct Job { int slot; int flags; uint64_t seq; bool detect; };
 
 struct GpuGroup {
     int device = 0;
@@ -53,13 +54,25 @@ struct GpuGroup {
     int rc[POOL_RING_MAX] = {};
     int valid[POOL_RING_MAX] = {};
     int has_mask[POOL_RING_MAX] = {};
+    int has_dmask[POOL_RING_MAX] = {};        // d_mask[slot] holds the slot's cleaned masks (kept for bgsb_pool_detect)
     std::string err[POOL_RING_MAX];
+    // bgsb_pool_detect: the records of this group's streams (filled by the driving thread), their moments query on the
+    // worker, on a stream of its own so that it runs beside the next frame sets
+    std::vector<MomRec> recs;
+    MomentBatch moments;
+    cudaStream_t s_det = nullptr;
+    cudaEvent_t ev_det = nullptr;
+    uint64_t det_seq = 0;                     // sequence number of the last detect job the worker has enqueued
+    int det_rc = 0;
+    std::string det_err;
 };
 
 }  // namespace
 
 struct bgsb_pool {
     int algo = 0, nstreams = 0, w = 0, h = 0, ring = 2, table_rows = 256;
+    int zero_border = 1;                             // the pipelines' "zeroBorder"
+    bool waited[POOL_RING_MAX] = {};                 // the slot's last submit has been waited for
     std::vector<GpuGroup *> groups;
     std::vector<int> group_of, index_in_group;      // per global stream
     uint64_t seq = 0;
@@ -79,6 +92,24 @@ static void worker_main(bgsb_pool *P, GpuGroup *G)
             j = G->jobs.front();
             G->jobs.pop_front();
         }
+        if (j.detect) {
+            // the slot's masks are complete (the caller waited for it) and stay until it is resubmitted
+            int rc = G->moments.reserve((int)G->recs.size());
+            if (!rc) {
+                memcpy(G->moments.h_rec, G->recs.data(), G->recs.size() * sizeof(MomRec));
+                rc = G->moments.enqueue(G->d_mask[j.slot], nullptr, P->w, P->h, (int)G->recs.size(), G->s_det);
+            }
+            if (!rc && cudaEventRecord(G->ev_det, G->s_det) != cudaSuccess) {
+                set_error("bgsb_pool_detect: cudaEventRecord -> %s", cudaGetErrorString(cudaGetLastError()));
+                rc = BGSB_ERR_CUDA;
+            }
+            {
+                std::lock_guard<std::mutex> lk(G->mu);
+                G->det_rc = rc; G->det_err = rc ? bgsb_last_error() : ""; G->det_seq = j.seq;
+            }
+            G->cv_done.notify_all();
+            continue;
+        }
         const int k = j.slot;
         const size_t S = G->streams.size();
         int rc = BGSB_OK, valid = 0;
@@ -97,7 +128,7 @@ static void worker_main(bgsb_pool *P, GpuGroup *G)
             if (fail(cudaEventRecord(G->ev_up[k], G->s_h2d), "record")) break;
             if (fail(cudaStreamWaitEvent(G->s_k, G->ev_up[k], 0), "wait(upload)")) break;
             int bgv = 0;
-            rc = bgsb_pipeline_process_dev(G->pipe, G->d_in[k], P->w, P->h, j.want_masks ? G->d_mask[k] : nullptr, nullptr, nullptr,
+            rc = bgsb_pipeline_process_dev(G->pipe, G->d_in[k], P->w, P->h, j.flags ? G->d_mask[k] : nullptr, nullptr, nullptr,
                                            &valid, &bgv, G->s_k);
             if (rc) { err = bgsb_last_error(); break; }
             if (fail(cudaEventRecord(G->ev_k[k], G->s_k), "record")) break;
@@ -110,7 +141,7 @@ static void worker_main(bgsb_pool *P, GpuGroup *G)
                 if (rc) { err = bgsb_last_error(); break; }
             }
             if (valid) {
-                if (j.want_masks && fail(cudaMemcpyAsync(G->h_mask[k], G->d_mask[k], S * P->mask_bytes, cudaMemcpyDeviceToHost, G->s_d2h), "download masks")) break;
+                if ((j.flags & BGSB_POOL_MASKS) && fail(cudaMemcpyAsync(G->h_mask[k], G->d_mask[k], S * P->mask_bytes, cudaMemcpyDeviceToHost, G->s_d2h), "download masks")) break;
                 if (fail(cudaMemcpyAsync(G->h_tab[k], G->d_tab[k], S * P->tab_ints * sizeof(int32_t), cudaMemcpyDeviceToHost, G->s_d2h), "download tables")) break;
             }
             if (fail(cudaEventRecord(G->ev_done[k], G->s_d2h), "record")) break;
@@ -118,7 +149,8 @@ static void worker_main(bgsb_pool *P, GpuGroup *G)
         } while (0);
         {
             std::lock_guard<std::mutex> lk(G->mu);
-            G->rc[k] = rc; G->err[k] = err; G->valid[k] = valid; G->has_mask[k] = valid && j.want_masks;
+            G->rc[k] = rc; G->err[k] = err; G->valid[k] = valid; G->has_mask[k] = valid && (j.flags & BGSB_POOL_MASKS);
+            G->has_dmask[k] = valid && j.flags;
             G->enq_seq[k] = j.seq;
         }
         G->cv_done.notify_all();
@@ -148,9 +180,30 @@ static void pool_free(bgsb_pool *P)
         if (G->s_h2d) cudaStreamDestroy(G->s_h2d);
         if (G->s_k) cudaStreamDestroy(G->s_k);
         if (G->s_d2h) cudaStreamDestroy(G->s_d2h);
+        if (G->s_det) cudaStreamDestroy(G->s_det);
+        if (G->ev_det) cudaEventDestroy(G->ev_det);
+        G->moments.release();
         delete G;
     }
     P->groups.clear();
+}
+
+// the table rings at P->table_rows rows per stream (create, and "tableRows" before the first submit)
+static int alloc_tables(bgsb_pool *P)
+{
+    P->tab_ints = (size_t)(P->table_rows + 1) * 8;
+    for (GpuGroup *G : P->groups) {
+        const size_t bytes = G->streams.size() * P->tab_ints * sizeof(int32_t);
+        BGSB_CUDA(cudaSetDevice(G->device));
+        for (int k = 0; k < P->ring; k++) {
+            if (G->h_tab[k]) cudaFreeHost(G->h_tab[k]);
+            cudaFree(G->d_tab[k]);
+            G->h_tab[k] = nullptr; G->d_tab[k] = nullptr;
+            BGSB_CUDA(cudaHostAlloc((void **)&G->h_tab[k], bytes, cudaHostAllocDefault));
+            BGSB_CUDA(cudaMalloc(&G->d_tab[k], bytes));
+        }
+    }
+    return BGSB_OK;
 }
 
 extern "C" {
@@ -164,7 +217,6 @@ int bgsb_pool_create(bgsb_pool **out, int algo, int nstreams, const int *devices
     bgsb_pool *P = new bgsb_pool();
     P->algo = algo; P->nstreams = nstreams; P->w = w; P->h = h; P->ring = ring;
     P->frame_bytes = (size_t)w * h * 3; P->mask_bytes = (size_t)w * h;
-    P->tab_ints = (size_t)(P->table_rows + 1) * 8;
     P->group_of.assign(nstreams, 0); P->index_in_group.assign(nstreams, 0);
     const int ng = std::min(ndevices, nstreams);
     int rc = BGSB_OK;
@@ -183,13 +235,13 @@ int bgsb_pool_create(bgsb_pool **out, int algo, int nstreams, const int *devices
         if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&G->s_h2d, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&G->s_k, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&G->s_d2h, cudaStreamNonBlocking);
+        if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&G->s_det, cudaStreamNonBlocking);
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&G->ev_det, cudaEventDisableTiming);
         for (int k = 0; k < ring && e == cudaSuccess; k++) {
             e = cudaHostAlloc((void **)&G->h_in[k], S * P->frame_bytes, cudaHostAllocDefault);
             if (e == cudaSuccess) e = cudaHostAlloc((void **)&G->h_mask[k], S * P->mask_bytes, cudaHostAllocDefault);
-            if (e == cudaSuccess) e = cudaHostAlloc((void **)&G->h_tab[k], S * P->tab_ints * sizeof(int32_t), cudaHostAllocDefault);
             if (e == cudaSuccess) e = cudaMalloc(&G->d_in[k], S * P->frame_bytes);
             if (e == cudaSuccess) e = cudaMalloc(&G->d_mask[k], S * P->mask_bytes);
-            if (e == cudaSuccess) e = cudaMalloc(&G->d_tab[k], S * P->tab_ints * sizeof(int32_t));
             if (e == cudaSuccess) e = cudaEventCreateWithFlags(&G->ev_up[k], cudaEventDisableTiming);
             if (e == cudaSuccess) e = cudaEventCreateWithFlags(&G->ev_k[k], cudaEventDisableTiming);
             if (e == cudaSuccess) e = cudaEventCreateWithFlags(&G->ev_done[k], cudaEventDisableTiming);
@@ -200,6 +252,7 @@ int bgsb_pool_create(bgsb_pool **out, int algo, int nstreams, const int *devices
             rc = BGSB_ERR_CUDA;
         }
     }
+    if (!rc) rc = alloc_tables(P);
     if (rc) { pool_free(P); delete P; return rc; }
     for (GpuGroup *G : P->groups) G->th = std::thread(worker_main, P, G);
     *out = P;
@@ -216,10 +269,17 @@ void bgsb_pool_destroy(bgsb_pool *P)
 int bgsb_pool_set_param(bgsb_pool *P, const char *key, double v)
 {
     BGSB_REQUIRE(P && key, "null");
+    if (std::string(key) == "tableRows") {
+        BGSB_REQUIRE(P->seq == 0, "tableRows: set it before the first submit");
+        BGSB_REQUIRE(v >= 1 && v <= (1 << 24), "tableRows in [1, 2^24]");
+        P->table_rows = (int)v;
+        return alloc_tables(P);
+    }
     for (GpuGroup *G : P->groups) {
         int rc = bgsb_pipeline_set_param(G->pipe, key, v);
         if (rc) return rc;
     }
+    if (std::string(key) == "zeroBorder") P->zero_border = (v != 0);
     return BGSB_OK;
 }
 
@@ -247,13 +307,15 @@ uint8_t *bgsb_pool_frame_buffer(bgsb_pool *P, int stream, int slot)
     return G->h_in[slot] + (size_t)P->index_in_group[stream] * P->frame_bytes;
 }
 
-int bgsb_pool_submit(bgsb_pool *P, int slot, int want_masks)
+int bgsb_pool_submit(bgsb_pool *P, int slot, int flags)
 {
     BGSB_REQUIRE(P && slot >= 0 && slot < P->ring, "slot index");
+    BGSB_REQUIRE((flags & ~(BGSB_POOL_MASKS | BGSB_POOL_DETECT)) == 0, "flags: BGSB_POOL_MASKS | BGSB_POOL_DETECT");
     const uint64_t seq = ++P->seq;
     P->want_seq[slot] = seq;
+    P->waited[slot] = false;
     for (GpuGroup *G : P->groups) {
-        { std::lock_guard<std::mutex> lk(G->mu); G->jobs.push_back(Job{slot, want_masks, seq}); }
+        { std::lock_guard<std::mutex> lk(G->mu); G->jobs.push_back(Job{slot, flags, seq, false}); }
         G->cv.notify_one();
     }
     return BGSB_OK;
@@ -274,6 +336,7 @@ int bgsb_pool_wait(bgsb_pool *P, int slot, int *valid)
         }
         BGSB_CUDA(cudaEventSynchronize(G->ev_done[slot]));
     }
+    P->waited[slot] = true;
     if (valid) *valid = all_valid;
     return BGSB_OK;
 }
@@ -302,6 +365,72 @@ int bgsb_pool_components(bgsb_pool *P, int stream, int slot, bgsb_component *out
         return BGSB_ERR_CAPACITY;
     }
     memcpy(out, t + 8, (size_t)cnt * sizeof(bgsb_component));
+    return BGSB_OK;
+}
+
+int bgsb_pool_detect(bgsb_pool *P, int slot, bgsb_blobdetector *const *bds, const bgsb_blob *const *old_blobs,
+                     const int *n_old, bgsb_blob *new_blobs, int *result, bgsb_blob *frame_blobs, int *n_frame, int *status)
+{
+    BGSB_REQUIRE(P && slot >= 0 && slot < P->ring, "slot index");
+    BGSB_REQUIRE(new_blobs && result && status, "null");
+    if (!P->waited[slot]) { set_error("bgsb_pool_detect: slot %d has not been waited for since its submit", slot); return BGSB_ERR_STATE; }
+    for (GpuGroup *G : P->groups) {
+        if (!G->valid[slot]) { set_error("bgsb_pool_detect: the slot holds no mask (plugin warm-up frame)"); return BGSB_ERR_STATE; }
+        if (!G->has_dmask[slot]) {
+            set_error("bgsb_pool_detect: slot %d was submitted without BGSB_POOL_DETECT", slot);
+            return BGSB_ERR_STATE;
+        }
+    }
+    int rc = detect_check(bds, P->nstreams, old_blobs, n_old, P->zero_border);
+    if (rc) return rc;
+    // (a) per stream from the tables on the host; the rectangles of a GPU's streams go to its worker as one query
+    const int N = P->nstreams;
+    std::vector<std::vector<int32_t>> rects(N);
+    int over = -1;
+    for (int s = 0; s < N; s++) {
+        GpuGroup *G = P->groups[P->group_of[s]];
+        const int32_t *t = G->h_tab[slot] + (size_t)P->index_in_group[s] * P->tab_ints;
+        status[s] = t[0] > P->table_rows ? BGSB_ERR_CAPACITY : BGSB_OK;
+        if (status[s]) { if (over < 0) over = s; continue; }
+        detect_rects(bds[s], reinterpret_cast<const bgsb_component *>(t + 8), t[0], P->w, P->h, rects[s]);
+    }
+    std::vector<int> first(N, 0);
+    for (GpuGroup *G : P->groups) {
+        G->recs.clear();
+        for (int s : G->streams) {
+            first[s] = (int)G->recs.size();
+            const std::vector<int32_t> &r = rects[s];
+            for (size_t i = 0; i < r.size(); i += 4)
+                G->recs.push_back(MomRec{P->index_in_group[s], r[i], r[i + 1], r[i + 2], r[i + 3], 0, 0, 0});
+        }
+    }
+    const uint64_t seq = ++P->seq;
+    for (GpuGroup *G : P->groups) {
+        { std::lock_guard<std::mutex> lk(G->mu); G->jobs.push_back(Job{slot, 0, seq, true}); }
+        G->cv.notify_one();
+    }
+    for (GpuGroup *G : P->groups) {
+        std::unique_lock<std::mutex> lk(G->mu);
+        G->cv_done.wait(lk, [&] { return G->det_seq >= seq; });
+        if (G->det_rc && !rc) { rc = G->det_rc; set_error("bgsb_pool_detect (device %d): %s", G->device, G->det_err.c_str()); }
+    }
+    if (rc) return rc;
+    for (GpuGroup *G : P->groups) BGSB_CUDA(cudaEventSynchronize(G->ev_det));
+    // (b) per stream
+    for (int s = 0; s < N; s++) {
+        if (status[s]) continue;
+        GpuGroup *G = P->groups[P->group_of[s]];
+        int n_new = 0;
+        detect_finish(bds[s], rects[s].data(), (int)rects[s].size() / 4,
+                      reinterpret_cast<const uint64_t *>(G->moments.h_mom) + 6 * first[s], P->w, P->h,
+                      old_blobs ? old_blobs[s] : nullptr, old_blobs ? n_old[s] : 0, new_blobs + s, 1, &n_new, result + s,
+                      frame_blobs ? frame_blobs + 10 * s : nullptr, 10, n_frame ? n_frame + s : nullptr);
+    }
+    if (over >= 0) {
+        set_error("bgsb_pool_detect: stream %d (and maybe others) has more components than \"tableRows\" = %d; its "
+                  "detector did not advance", over, P->table_rows);
+        return BGSB_ERR_CAPACITY;
+    }
     return BGSB_OK;
 }
 

@@ -13,7 +13,7 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .blobs import _ops
+from .blobs import _ops, detect_streams
 
 
 class ForegroundPipeline:
@@ -80,6 +80,14 @@ class ForegroundPipeline:
         capi.check(capi.lib().bgsb_pipeline_rect_moments(self._h, stream_index, flat.ctypes.data_as(capi.i32p),
                                                          len(rects), out))
         return [[int(out[6 * i + j]) for j in range(6)] for i in range(len(rects))]
+
+    def detect(self, detectors, old_blobs=None):
+        """DetectNewBlob for every stream of the last frame on the labelling already done: detectors[s] is stream s's
+        blobs.CvBlobDetectorCC, old_blobs[s] its tracked blobs [(x, y, w, h)] (None: none anywhere).
+        -> per stream (result, new_blob | None, frame_blobs)."""
+        if len(detectors) != self.nstreams:
+            raise ValueError("one detector per stream")
+        return detect_streams(capi.lib().bgsb_pipeline_detect, (self._h,), detectors, old_blobs)
 
     def export_mog2_state(self, stream_index=0):
         if self.algo != capi.ALGO_MOG2 or self._shape is None:

@@ -17,7 +17,7 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .blobs import _ops
+from .blobs import _ops, detect_streams
 
 
 def shard_streams(nstreams: int, world_size: int, rank: int):
@@ -44,6 +44,8 @@ class StreamPool:
         pool.submit(slot)                                # every stream's frame of `slot` is in place
         valid = pool.wait(slot)
         blobs = pool.components(s, slot)                 # bounding boxes / areas / external flags of stream s
+
+    With submit(slot, detect=True), detect(slot, detectors, old_blobs) then runs DetectNewBlob for every stream.
     """
 
     def __init__(self, algo, nstreams, w, h, devices=None, ring=2, morph=None, **params):
@@ -90,8 +92,10 @@ class StreamPool:
         buf = (C.c_uint8 * (self.h * self.w * 3)).from_address(p)
         return np.frombuffer(buf, dtype=np.uint8).reshape(self.h, self.w, 3)
 
-    def submit(self, slot, want_masks=False):
-        capi.check(capi.lib().bgsb_pool_submit(self._h, slot, int(want_masks)))
+    def submit(self, slot, want_masks=False, detect=False):
+        """want_masks: download the cleaned masks (mask()); detect: keep them on the device for detect()."""
+        flags = (capi.POOL_MASKS if want_masks else 0) | (capi.POOL_DETECT if detect else 0)
+        capi.check(capi.lib().bgsb_pool_submit(self._h, slot, flags))
 
     def wait(self, slot):
         v = C.c_int(0)
@@ -104,6 +108,15 @@ class StreamPool:
             return None
         buf = (C.c_uint8 * (self.h * self.w)).from_address(p)
         return np.frombuffer(buf, dtype=np.uint8).reshape(self.h, self.w)
+
+    def detect(self, slot, detectors, old_blobs=None):
+        """DetectNewBlob for every stream of a waited-for slot submitted with detect=True: detectors[s] is stream s's
+        blobs.CvBlobDetectorCC, old_blobs[s] its tracked blobs [(x, y, w, h)] (None: none anywhere).  -> per stream
+        (result, new_blob | None, frame_blobs), or None for a stream with more than table_rows components (its detector
+        did not advance; raise "tableRows")."""
+        if len(detectors) != self.nstreams:
+            raise ValueError("one detector per stream")
+        return detect_streams(capi.lib().bgsb_pool_detect, (self._h, slot), detectors, old_blobs)
 
     def components(self, stream, slot):
         n = C.c_int(0)
