@@ -65,6 +65,18 @@ enum {
     BGSB_ALGO_SIGMA_DELTA = 35                    /* ustc_bgs.cpp:62  sibling plugin (BL package); first frame: no outputs */
 };
 
+/* Values of the "inputFormat" parameter (bgsb_set_param): the layout of the frames a context's calls take.
+ *   BGSB_INPUT_BGR  : interleaved BGR, 3 bytes per pixel (default).
+ *   BGSB_INPUT_NV12 : YUV 4:2:0 as NVDEC, V4L2 and most camera SDKs produce it: h rows of w Y bytes, then h/2 rows of w
+ *                     bytes of interleaved U,V; on host paths both kinds of row sit `stride` bytes apart.
+ *   BGSB_INPUT_I420 : YUV 4:2:0 planar (ffmpeg's AV_PIX_FMT_YUV420P): the Y plane (w x h), the U plane (w/2 x h/2), the V
+ *                     plane, densely packed; on host paths `stride` must equal w.
+ * Both are one 8-bit image of 3h/2 rows of w bytes, the cv::Mat that cv::cvtColor(COLOR_YUV2BGR_NV12 / _I420) reads; w
+ * and h must be even.  Device buffers are dense: [nstreams][3h/2][w], and [nstreams][T][3h/2][w] for batches.  The
+ * library converts each frame on the device to exactly the BGR image cv::cvtColor gives (BT.601, limited range,
+ * 20-bit fixed point) and runs the plugin on it, so every result equals that of the BGR path fed cv::cvtColor's output. */
+enum { BGSB_INPUT_BGR = 0, BGSB_INPUT_NV12 = 1, BGSB_INPUT_I420 = 2 };
+
 typedef struct bgsb_ctx bgsb_ctx;
 
 /* ---------------------------------------------------------------------------------------
@@ -139,7 +151,14 @@ BGSB_API int bgsb_reset(bgsb_ctx *ctx);
  * 1 = the caller promises that the device frame given to a call stays valid and unmodified until the next call (FD)
  * / the next two calls (WMV, WMM) have completed, so the previous-frame history is read from those buffers and never
  * copied (the reference's img_input_prev members, FrameDifferenceBGS.cpp:58, WeightedMovingVarianceBGS.cpp:113-114):
- * FD moves 7 B/px instead of 10, WMV 10 instead of 16.  Single frames, or batches on a single-stream context. */
+ * FD moves 7 B/px instead of 10, WMV 10 instead of 16.  Single frames, or batches on a single-stream context;
+ * "inputFormat" (default BGSB_INPUT_BGR): BGSB_INPUT_NV12 / BGSB_INPUT_I420 make every entry point (bgsb_process,
+ * bgsb_submit, bgsb_process_fanout, bgsb_process_dev, bgsb_process_batch_dev, the pipeline and the pool) take YUV 4:2:0
+ * frames (see the enum above).  The host paths upload 1.5 B/px instead of 3 and convert on the device into the buffer
+ * the BGR upload would fill; the device paths convert into a library-owned scratch on the caller's stream first.  The
+ * model and the history are kept as BGR, so the format may change between calls.  BGSB_ERR_ARG for an odd w or h, an
+ * I420 host frame with stride != w, and together with "retainInput" (the converted frames are the library's, so the
+ * caller's buffers cannot serve as the history).  Fan-out contexts must share one format. */
 BGSB_API int bgsb_set_param(bgsb_ctx *ctx, const char *key, double value);
 BGSB_API int bgsb_get_param(bgsb_ctx *ctx, const char *key, double *value);
 
@@ -372,7 +391,8 @@ BGSB_API int bgsb_pipeline_detect(bgsb_pipeline *p, bgsb_blobdetector *const *bd
  * one camera; the pool runs that loop for many: stream s lives on devices[s % ndevices], each GPU has one host worker
  * thread, one bgsb_pipeline over its streams, and `ring` slots of page-locked frame / mask / table buffers on three CUDA
  * streams, so that slot k+1 uploads while slot k computes and slot k-1 downloads.  Streams never exchange data.
- *   capture side : write frame t of stream s into bgsb_pool_frame_buffer(pool, s, t % ring)   (h*w*3 bytes, dense BGR)
+ *   capture side : write frame t of stream s into bgsb_pool_frame_buffer(pool, s, t % ring)   (h*w*3 bytes, dense BGR;
+ *                  with "inputFormat" NV12 / I420: h*w*3/2 bytes, the dense 3h/2 x w YUV image)
  *   bgsb_pool_submit(pool, slot, flags)      : every stream's frame of that slot is ready; returns at once
  *   bgsb_pool_wait(pool, slot, &valid)       : that slot's results are on the host; valid = 0 while the plugin warms up
  *   bgsb_pool_mask / bgsb_pool_components    : the cleaned {0,255} mask (if asked for) and the component table
@@ -390,7 +410,9 @@ BGSB_API int bgsb_pool_create(bgsb_pool **out, int algo, int nstreams, const int
                               int ring);
 BGSB_API void bgsb_pool_destroy(bgsb_pool *pool);
 /* As bgsb_pipeline_set_param / bgsb_pipeline_set_morph, applied to every GPU's pipeline; call before the first submit.
- * The pool's own key "tableRows" (default 256) sets how many components per stream and frame come back to the host. */
+ * The pool's own key "tableRows" (default 256) sets how many components per stream and frame come back to the host.
+ * "inputFormat" (BGSB_INPUT_*) is accepted before the first submit only (BGSB_ERR_ARG after it): it resizes the frame
+ * buffers and the uploads to h*w*3/2 bytes per stream, and each GPU's pipeline converts its streams' frames. */
 BGSB_API int bgsb_pool_set_param(bgsb_pool *pool, const char *key, double value);
 BGSB_API int bgsb_pool_set_morph(bgsb_pool *pool, const int *ops, int nops);
 BGSB_API int bgsb_pool_device_of(bgsb_pool *pool, int stream, int *device);

@@ -17,16 +17,22 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJDIR = os.path.join(HERE, "_obj")
 LIB = os.path.join(HERE, "libbgsb200.so")
-SOURCES = ["capi.cu", "simple_bgs.cu", "mog2.cu", "mog2_t1.cu", "dpz.cu", "dp_simple.cu", "synth.cu", "morph.cu", "ccl.cu", "blobdetect.cu", "pipeline.cu", "pool.cu"]
+SOURCES = ["capi.cu", "simple_bgs.cu", "mog2.cu", "mog2_t1.cu", "dpz.cu", "dp_simple.cu", "synth.cu", "morph.cu", "ccl.cu", "blobdetect.cu", "pipeline.cu", "pool.cu",
+           os.path.join("ingest", "yuv420.cu")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-fmad=false",
          "-Xcompiler", "-fPIC,-fvisibility=hidden", "-Xptxas", "-v"]
 
 
 def _deps():
-    d = [os.path.join(CSRC, f) for f in os.listdir(CSRC)]
+    d = [os.path.join(base, f) for base, _, names in os.walk(CSRC) for f in names]
     d.append(os.path.join(HERE, "..", "include", "bgsb200.h"))
     return d
+
+
+def _obj_name(src):
+    """ingest/yuv420.cu -> ingest__yuv420.o: one flat object directory for sources in subdirectories"""
+    return src.replace(os.sep, "__").replace(".cu", ".o")
 
 
 def needs_build():
@@ -43,14 +49,14 @@ def build(force=False, verbose=False, instrument=False):
         return LIB
     os.makedirs(OBJDIR, exist_ok=True)
     srcs = [s for s in SOURCES if os.path.exists(os.path.join(CSRC, s))]
-    keep = {s.replace(".cu", ".o") for s in srcs} | {"ptxas.log"}
+    keep = {_obj_name(s) for s in srcs} | {"ptxas.log"}
     for f in os.listdir(OBJDIR):                 # objects of sources that no longer exist must not travel to the GPU box
         if f not in keep:
             os.remove(os.path.join(OBJDIR, f))
     flags = FLAGS + (["-DBGSB_INSTRUMENT"] if instrument else [])
 
     def cc(src):
-        obj = os.path.join(OBJDIR, src.replace(".cu", ".o"))
+        obj = os.path.join(OBJDIR, _obj_name(src))
         cmd = [NVCC, *flags, "-c", os.path.join(CSRC, src), "-o", obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:

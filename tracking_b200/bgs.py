@@ -24,10 +24,35 @@ def _ptr(a):
     return C.c_void_p(a.ctypes.data)
 
 
+def yuv_frame(img, fmt, nstreams=1):
+    """Check a YUV 4:2:0 frame for "inputFormat" fmt (capi.INPUT_NV12 / INPUT_I420): the (3h/2, w) uint8 image that
+    cv::cvtColor reads, with a leading stream axis for a group.  -> (array with unit-stride rows, h, w, grouped); NV12
+    rows may be padded (the row stride is passed on), I420 planes are made dense."""
+    if fmt not in (capi.INPUT_NV12, capi.INPUT_I420):
+        raise ValueError("inputFormat %r is not a YUV format" % (fmt,))
+    img = np.asarray(img)
+    grouped = img.ndim == 3
+    if img.dtype != np.uint8 or img.ndim not in (2, 3):
+        raise ValueError("YUV 4:2:0 input takes (3h/2, w) uint8 frames (a stream group: (nstreams, 3h/2, w))")
+    if grouped and img.shape[0] != nstreams:
+        raise ValueError("expected %d frames" % nstreams)
+    if not grouped and nstreams != 1:
+        raise ValueError("stream group needs [nstreams, 3h/2, w]")
+    rows, w = img.shape[-2], img.shape[-1]
+    if rows == 0 or w == 0 or rows % 3 or w % 2:         # (3h/2 rows: h = 2 rows / 3 is even whenever 3 divides rows)
+        raise ValueError("YUV 4:2:0 frames have 3h/2 rows of w bytes with w and h even (got %d x %d)" % (rows, w))
+    h = 2 * rows // 3
+    dense = img.strides[-1] == 1 and (fmt == capi.INPUT_NV12 or img.strides[-2] == w)
+    if not dense or (grouped and img.strides[0] != img.strides[1] * rows):
+        img = np.ascontiguousarray(img)
+    return img, h, w, grouped
+
+
 class _Plugin:
     ALGO = None
     PARAMS = ()
     BG_CHANNELS = 3            # channels of img_bgmodel (AdaptiveSelectiveBackgroundLearning: 1)
+    input_format = capi.INPUT_BGR     # "inputFormat": the layout process / submit / process_fanout take
 
     def __init__(self, device=0, nstreams=1, **params):
         self._h = C.c_void_p()
@@ -39,6 +64,8 @@ class _Plugin:
     # -- parameters: XML key names of saveConfig/loadConfig ---------------------------------
     def set(self, key, value):
         capi.check(capi.lib().bgsb_set_param(self._h, key.encode(), float(value)))
+        if key == "inputFormat":
+            self.input_format = int(value)
 
     def get(self, key):
         v = C.c_double()
@@ -67,22 +94,26 @@ class _Plugin:
 
     # -- IBGS::process, host buffers -------------------------------------------------------
     def process(self, img_input, want_bg=True):
-        """img_input: HxWx3 uint8 BGR (a group takes nstreams x H x W x 3).
-        Returns (img_output | None, img_bgmodel | None)."""
+        """img_input: HxWx3 uint8 BGR (a group takes nstreams x H x W x 3); with "inputFormat" NV12 / I420 the
+        (3h/2) x W YUV image (a group: nstreams x 3h/2 x W).  Returns (img_output | None, img_bgmodel | None)."""
         if img_input is None or img_input.size == 0:      # `if(img_input.empty()) return;`
             return None, None
-        img = np.asarray(img_input)
-        if img.dtype != np.uint8 or img.shape[-1] != 3:
-            raise ValueError("plugins take BGR 8UC3 frames")
-        grouped = img.ndim == 4
-        if grouped and img.shape[0] != self.nstreams:
-            raise ValueError("expected %d frames" % self.nstreams)
-        if not grouped and self.nstreams != 1:
-            raise ValueError("stream group needs [nstreams,H,W,3]")
-        h, w = img.shape[-3], img.shape[-2]
-        if img.strides[-1] != 1 or img.strides[-2] != 3 or (grouped and img.strides[0] != img.strides[1] * h):
-            img = np.ascontiguousarray(img)
-        stride = img.strides[-3]
+        if self.input_format != capi.INPUT_BGR:
+            img, h, w, grouped = yuv_frame(img_input, self.input_format, self.nstreams)
+            stride = img.strides[-2]
+        else:
+            img = np.asarray(img_input)
+            if img.dtype != np.uint8 or img.shape[-1] != 3:
+                raise ValueError("plugins take BGR 8UC3 frames")
+            grouped = img.ndim == 4
+            if grouped and img.shape[0] != self.nstreams:
+                raise ValueError("expected %d frames" % self.nstreams)
+            if not grouped and self.nstreams != 1:
+                raise ValueError("stream group needs [nstreams,H,W,3]")
+            h, w = img.shape[-3], img.shape[-2]
+            if img.strides[-1] != 1 or img.strides[-2] != 3 or (grouped and img.strides[0] != img.strides[1] * h):
+                img = np.ascontiguousarray(img)
+            stride = img.strides[-3]
         lead = (self.nstreams,) if grouped else ()
         fg = np.empty(lead + (h, w), np.uint8)
         bgshape = (h, w, 3) if self.BG_CHANNELS == 3 else (h, w)
@@ -98,18 +129,26 @@ class _Plugin:
         """Queue one frame (bgsb_submit): like process(), but returns once the work is enqueued; the upload of the
         next frame overlaps this frame's download.  img_input / fg_out / bg_out are caller-owned C-contiguous uint8
         arrays (page-locked ones from pinned_empty() to really overlap) that must stay untouched until wait().
+        With "inputFormat" NV12 / I420, img_input is the C-contiguous (3h/2) x W YUV image.
         Returns (fg_valid, bg_valid): whether fg_out / bg_out will be written for this frame."""
         img = np.asarray(img_input)
-        if img.dtype != np.uint8 or img.ndim != 3 or img.shape[-1] != 3 or not img.flags.c_contiguous:
-            raise ValueError("submit takes one C-contiguous BGR 8UC3 frame")
-        h, w = img.shape[:2]
+        if self.input_format != capi.INPUT_BGR:
+            if img.ndim != 2 or not img.flags.c_contiguous:
+                raise ValueError("submit takes one C-contiguous (3h/2, w) YUV 4:2:0 frame")
+            img, h, w, _ = yuv_frame(img, self.input_format)
+            stride = w
+        else:
+            if img.dtype != np.uint8 or img.ndim != 3 or img.shape[-1] != 3 or not img.flags.c_contiguous:
+                raise ValueError("submit takes one C-contiguous BGR 8UC3 frame")
+            h, w = img.shape[:2]
+            stride = w * 3
         if fg_out.dtype != np.uint8 or fg_out.shape != (h, w) or not fg_out.flags.c_contiguous:
             raise ValueError("fg_out must be a C-contiguous HxW uint8 array")
         bgshape = (h, w, 3) if self.BG_CHANNELS == 3 else (h, w)
         if bg_out is not None and (bg_out.dtype != np.uint8 or bg_out.shape != bgshape or not bg_out.flags.c_contiguous):
             raise ValueError("bg_out must be a C-contiguous uint8 array of shape %r" % (bgshape,))
         fv, bv = C.c_int(0), C.c_int(0)
-        capi.check(capi.lib().bgsb_submit(self._h, _ptr(img), w, h, w * 3, _ptr(fg_out), w,
+        capi.check(capi.lib().bgsb_submit(self._h, _ptr(img), w, h, stride, _ptr(fg_out), w,
                                           _ptr(bg_out) if bg_out is not None else None, self.BG_CHANNELS * w,
                                           C.byref(fv), C.byref(bv)))
         self._keep = getattr(self, "_keep", [])
@@ -123,6 +162,7 @@ class _Plugin:
 
     # -- device buffers (torch tensors or raw pointers) -----------------------------------------
     def process_dev(self, d_bgr, w, h, d_fg, d_bg=None, stream=0):
+        """d_bgr: device pointer to [nstreams][h][w][3] (with "inputFormat" NV12 / I420: [nstreams][3h/2][w])."""
         fv, bv = C.c_int(0), C.c_int(0)
         capi.check(capi.lib().bgsb_process_dev(self._h, C.c_void_p(d_bgr), w, h, C.c_void_p(d_fg),
                                                C.c_void_p(d_bg) if d_bg else None,
@@ -130,6 +170,7 @@ class _Plugin:
         return bool(fv.value), bool(bv.value)
 
     def process_batch_dev(self, d_frames, T, w, h, d_fg, d_bg=None, bg_last_only=False, stream=0):
+        """d_frames: device pointer to [nstreams][T][h][w][3] (with "inputFormat" NV12 / I420: [nstreams][T][3h/2][w])."""
         first, bv = C.c_int(0), C.c_int(0)
         capi.check(capi.lib().bgsb_process_batch_dev(self._h, C.c_void_p(d_frames), T, w, h, C.c_void_p(d_fg),
                                                      C.c_void_p(d_bg) if d_bg else None, int(bg_last_only),
@@ -264,15 +305,20 @@ def pinned_empty(shape, write_combined=False):
 
 def process_fanout(plugins, img_input, want_bg=True):
     """FrameProcessor::process (FrameProcessor.cpp:169-215): every plugin on the same frame, one upload.
-    Returns [(img_output | None, img_bgmodel | None), ...] exactly as plugin.process(img_input) would for each."""
+    Returns [(img_output | None, img_bgmodel | None), ...] exactly as plugin.process(img_input) would for each.
+    With "inputFormat" NV12 / I420 (the same on every plugin) img_input is the (3h/2) x W YUV image."""
     if img_input is None or img_input.size == 0:
         return [(None, None) for _ in plugins]
-    img = np.asarray(img_input)
-    if img.dtype != np.uint8 or img.ndim != 3 or img.shape[-1] != 3:
-        raise ValueError("fan-out takes one BGR 8UC3 frame")
-    if img.strides[-1] != 1 or img.strides[-2] != 3:
-        img = np.ascontiguousarray(img)
-    h, w = img.shape[:2]
+    fmt = plugins[0].input_format if plugins else capi.INPUT_BGR
+    if fmt != capi.INPUT_BGR:
+        img, h, w, _ = yuv_frame(img_input, fmt)
+    else:
+        img = np.asarray(img_input)
+        if img.dtype != np.uint8 or img.ndim != 3 or img.shape[-1] != 3:
+            raise ValueError("fan-out takes one BGR 8UC3 frame")
+        if img.strides[-1] != 1 or img.strides[-2] != 3:
+            img = np.ascontiguousarray(img)
+        h, w = img.shape[:2]
     n = len(plugins)
     fgs = [np.empty((h, w), np.uint8) for _ in plugins]
     bgs = [np.empty((h, w, 3) if p.BG_CHANNELS == 3 else (h, w), np.uint8) if want_bg else None for p in plugins]

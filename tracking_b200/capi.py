@@ -20,6 +20,7 @@ ALGO_DP_PRATI_MEDIOD = 14
 ALGO_SIGMA_DELTA = 35
 MORPH_ERODE, MORPH_DILATE = 0, 1
 POOL_MASKS, POOL_DETECT = 1, 2
+INPUT_BGR, INPUT_NV12, INPUT_I420 = 0, 1, 2                            # "inputFormat" (BGSB_INPUT_*)
 
 
 class BgsbError(RuntimeError):

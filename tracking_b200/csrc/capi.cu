@@ -161,6 +161,12 @@ struct bgsb_ctx {
     bool last_stream_set = false;
     cudaEvent_t ev_order = nullptr;
     int retain_input = 0;      // device path, FD / WMV / WMM: the caller's frames stay valid -> no history write-back
+    // "inputFormat": BGR, or YUV 4:2:0 frames (NV12 / I420) that ingest/yuv420.cu converts to BGR before the plugin runs;
+    // the model and the history stay BGR, so the format may change between calls
+    int input_format = BGSB_INPUT_BGR;
+    uint8_t *d_yuv = nullptr;             // host paths: the uploaded YUV frames [S][3h/2][w] (fan-out: the first context's)
+    uint8_t *d_conv = nullptr;            // device paths: the converted frames [S][T][h][w][3]
+    size_t d_conv_bytes = 0;
     // WMV quiet-group shortcut: wmv_bound[ew][r] = largest standard-deviation byte over all triples of range r for the
     // weight set ew (computed once per weight set on the device, launch_wmv_bound_table); wmv_quiet 0 switches it off
     int wmv_quiet = 1;
@@ -186,6 +192,7 @@ static void free_staging(bgsb_ctx *c)
     cudaFree(c->d_bg); c->d_bg = nullptr;
     cudaFree(c->d_fg2); c->d_fg2 = nullptr;
     cudaFree(c->d_bg2); c->d_bg2 = nullptr;
+    cudaFree(c->d_yuv); c->d_yuv = nullptr;
 }
 
 static void free_buffers(bgsb_ctx *c)
@@ -196,6 +203,7 @@ static void free_buffers(bgsb_ctx *c)
     for (int i = 0; i < 2; i++) { cudaFree(c->d_hist[i]); c->d_hist[i] = nullptr; c->hist_ptr[i] = nullptr; }
     free_staging(c);
     cudaFree(c->d_fan); c->d_fan = nullptr; c->d_fan_bytes = 0;
+    cudaFree(c->d_conv); c->d_conv = nullptr; c->d_conv_bytes = 0;
     cudaFree(c->d_prati); c->d_prati = nullptr; c->prati_bytes = 0; c->prati_n = c->prati_pos = 0;
     c->w = c->h = c->npx = 0; c->pstride = 0;
     c->nframes = 0; c->mog2_epoch = 0; c->have_hist = 0; c->ring_pos = 0;
@@ -276,6 +284,61 @@ static cudaError_t copy_rows(void *dst, size_t dpitch, const void *src, size_t s
 {
     if (dpitch == width && spitch == width) return cudaMemcpyAsync(dst, src, width * rows, kind, st);
     return cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, st);
+}
+
+// ---- YUV 4:2:0 input -------------------------------------------------------------------------------
+// The layout cv::cvtColor(COLOR_YUV2BGR_NV12 / _I420) reads: one 8-bit image of 3h/2 rows of w bytes.  NV12: h Y rows,
+// then h/2 rows of interleaved U,V; I420: the Y plane, the U plane (w/2 x h/2), the V plane, densely packed.  Host
+// frames have `stride` bytes between rows (I420: stride == w); device frames are dense, [frames][3h/2][w].
+static int check_yuv_frame(int fmt, int w, int h, size_t stride)
+{
+    BGSB_REQUIRE(w > 0 && h > 0 && w % 2 == 0 && h % 2 == 0, "YUV 4:2:0 input (inputFormat NV12 / I420) needs an even width and height");
+    BGSB_REQUIRE(stride >= (size_t)w, "stride smaller than a row");
+    BGSB_REQUIRE(fmt != BGSB_INPUT_I420 || stride == (size_t)w, "I420 frames are dense planes: stride must equal w");
+    return BGSB_OK;
+}
+
+// Rows [r0, r0 + nr) (r0, nr even) of `nframes` dense device YUV frames at src -> the same rows of dense BGR frames at dst.
+static int convert_yuv(int fmt, const uint8_t *src, int w, int h, int r0, int nr, int nframes, uint8_t *dst, cudaStream_t st)
+{
+    const size_t W = (size_t)w, H = (size_t)h;
+    Yuv420Launch L;
+    memset(&L, 0, sizeof(L));
+    L.y = src + r0 * W; L.y_pitch = W;
+    if (fmt == BGSB_INPUT_NV12) {
+        L.u = src + (H + r0 / 2) * W; L.c_pitch = W;
+    } else {
+        L.u = src + H * W + (r0 / 2) * (W / 2); L.v = L.u + (H / 2) * (W / 2); L.c_pitch = W / 2; L.planar = 1;
+    }
+    L.src_frame_stride = H * W * 3 / 2;
+    L.bgr = dst + r0 * W * 3; L.dst_frame_stride = H * W * 3;
+    L.w = w; L.rows = nr; L.nframes = nframes;
+    return launch_yuv420_to_bgr(L, st);
+}
+
+// Host rows [r0, r0 + nr) of `nframes` YUV frames stacked `stride`-apart rows -> the dense device staging at dst.  A band
+// (r0, nr) != (0, h) is one frame's Y rows and chroma rows; I420's planes are dense, so each plane's band is one span.
+static cudaError_t upload_yuv(int fmt, uint8_t *dst, const uint8_t *src, size_t stride, int w, int h, int r0, int nr,
+                              int nframes, cudaStream_t st)
+{
+    const size_t W = (size_t)w, H = (size_t)h;
+    if (r0 == 0 && nr == h) return copy_rows(dst, W, src, stride, W, (size_t)nframes * H * 3 / 2, cudaMemcpyHostToDevice, st);
+    cudaError_t e = copy_rows(dst + r0 * W, W, src + r0 * stride, stride, W, nr, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return e;
+    if (fmt == BGSB_INPUT_NV12)
+        return copy_rows(dst + (H + r0 / 2) * W, W, src + (H + r0 / 2) * stride, stride, W, nr / 2, cudaMemcpyHostToDevice, st);
+    const size_t q = W / 2, off = H * W + (r0 / 2) * q, n = (nr / 2) * q;
+    e = cudaMemcpyAsync(dst + off, src + off, n, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return e;
+    return cudaMemcpyAsync(dst + off + (H / 2) * q, src + off + (H / 2) * q, n, cudaMemcpyHostToDevice, st);
+}
+
+static int ensure_yuv_staging(bgsb_ctx *c)
+{
+    if (c->d_yuv) return BGSB_OK;
+    const cudaError_t e = cudaMalloc(&c->d_yuv, (size_t)c->nstreams * c->npx * 3 / 2);
+    if (e != cudaSuccess) return staging_fail(c, e);
+    return BGSB_OK;
 }
 
 // Launch the kernels that advance the model by T frames that sit in device memory, for pixels [p0, p0+pcount) of the
@@ -636,11 +699,15 @@ static int drain(bgsb_ctx *c)
 }
 
 // Arguments of bgsb_process / bgsb_submit: one frame, or a group's frames stacked.
-static int check_host_frame(const bgsb_ctx *c, const uint8_t *bgr, int w, size_t stride, const uint8_t *fg,
+static int check_host_frame(const bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, const uint8_t *fg,
                             size_t fg_stride, const uint8_t *bg, size_t bg_stride)
 {
     BGSB_REQUIRE(c && bgr && fg, "null");
-    BGSB_REQUIRE(stride >= (size_t)w * 3 && fg_stride >= (size_t)w, "stride smaller than a row");
+    if (c->input_format != BGSB_INPUT_BGR) {
+        int rc = check_yuv_frame(c->input_format, w, h, stride);
+        if (rc) return rc;
+    }
+    BGSB_REQUIRE(stride >= (size_t)w * (c->input_format == BGSB_INPUT_BGR ? 3 : 1) && fg_stride >= (size_t)w, "stride smaller than a row");
     BGSB_REQUIRE(!bg || bg_stride >= (size_t)w * c->pi->bg_channels, "bg stride smaller than a row");
     return BGSB_OK;
 }
@@ -788,7 +855,18 @@ int bgsb_set_param(bgsb_ctx *c, const char *key, double v)
     else if (k == "shadowValue") c->shadow_value = (int)v;
     else if (k == "shadowThreshold") c->tau = (float)v;
     else if (k == "hostBands") { BGSB_REQUIRE(v >= 1 && v <= 8, "hostBands in [1,8]"); c->host_bands = (int)v; c->host_bands_auto = false; }
-    else if (k == "retainInput") c->retain_input = (v != 0);
+    else if (k == "retainInput") {
+        BGSB_REQUIRE(v == 0 || c->input_format == BGSB_INPUT_BGR, "retainInput cannot be combined with a YUV inputFormat: the "
+                     "converted frames are the library's, so the caller's buffers cannot serve as the history");
+        c->retain_input = (v != 0);
+    }
+    else if (k == "inputFormat") {
+        BGSB_REQUIRE(v == BGSB_INPUT_BGR || v == BGSB_INPUT_NV12 || v == BGSB_INPUT_I420,
+                     "inputFormat is 0 (BGSB_INPUT_BGR), 1 (BGSB_INPUT_NV12) or 2 (BGSB_INPUT_I420)");
+        BGSB_REQUIRE(v == BGSB_INPUT_BGR || !c->retain_input, "a YUV inputFormat cannot be combined with retainInput: the "
+                     "converted frames are the library's, so the caller's buffers cannot serve as the history");
+        c->input_format = (int)v;
+    }
     else if (k == "quietGroups") c->wmv_quiet = (v != 0);
     else if (k == "trace") c->trace = (v != 0);
 #ifdef BGSB_INSTRUMENT
@@ -846,6 +924,7 @@ int bgsb_get_param(bgsb_ctx *c, const char *key, double *v)
     else if (k == "kernelVariant") *v = c->mog2_variant;
     else if (k == "hostBands") *v = c->host_bands;
     else if (k == "retainInput") *v = c->retain_input;
+    else if (k == "inputFormat") *v = c->input_format;
     else if (k == "quietGroups") *v = c->wmv_quiet;
     else if (k == "trace") *v = c->trace;
     else if (k == "ablTable") *v = c->abl_table;
@@ -904,17 +983,35 @@ static int process_batch_impl(bgsb_ctx *c, const uint8_t *d_frames, int T, int w
 {
     if (int drc = drain(c)) return drc;
     BGSB_REQUIRE(T >= 1, "T >= 1");
+    const bool yuv = c->input_format != BGSB_INPUT_BGR;
+    if (yuv) {
+        int rc = check_yuv_frame(c->input_format, w, h, (size_t)w);
+        if (rc) return rc;
+    }
     BGSB_CUDA(cudaSetDevice(c->device));
     int rc = ensure_geometry(c, w, h);
     if (rc) return rc;
     rc = order_after_previous(c, (cudaStream_t)stream);
     if (rc) return rc;
     latch_first_frame(c);
+    if (yuv) {
+        // the caller's YUV frames become BGR frames in a library-owned scratch, on the caller's stream; the plugin then
+        // runs on the scratch exactly as on BGR frames, writing its history back (the scratch is reused by the next call)
+        const size_t need = (size_t)c->nstreams * T * c->npx * 3;
+        if (c->d_conv_bytes < need) {
+            cudaFree(c->d_conv); c->d_conv = nullptr; c->d_conv_bytes = 0;
+            BGSB_CUDA(cudaMalloc(&c->d_conv, need));
+            c->d_conv_bytes = need;
+        }
+        rc = convert_yuv(c->input_format, d_frames, w, h, 0, h, c->nstreams * T, c->d_conv, (cudaStream_t)stream);
+        if (rc) return rc;
+        d_frames = c->d_conv;
+    }
     int64_t first = std::max<int64_t>(0, c->pi->warmup - c->nframes);
     if (first_fg_valid) *first_fg_valid = (int)std::min<int64_t>(first, T);
     const bool has_bg = c->pi->writes_bg;
     if (bg_valid) *bg_valid = has_bg && d_bg && (first < T);
-    if (c->retain_input && c->pi->ring_history && (T == 1 || c->nstreams == 1)) {
+    if (c->retain_input && !yuv && c->pi->ring_history && (T == 1 || c->nstreams == 1)) {
         // "retainInput": the caller keeps the last one (FD) / two (WMV, WMM) frame buffers valid and unmodified, so
         // the history IS those buffers -- as in the host path's upload ring -- and nothing is written back:
         // FD moves its 7 algorithmic bytes per pixel, WMV its 10 (SURVEY 8d).
@@ -946,7 +1043,7 @@ int bgsb_process_dev(bgsb_ctx *c, const uint8_t *d_bgr, int w, int h, uint8_t *d
 int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, uint8_t *fg, size_t fg_stride,
                  uint8_t *bg, size_t bg_stride, int *fg_valid, int *bg_valid)
 {
-    int rc = check_host_frame(c, bgr, w, stride, fg, fg_stride, bg, bg_stride);
+    int rc = check_host_frame(c, bgr, w, h, stride, fg, fg_stride, bg, bg_stride);
     if (rc) return rc;
     BGSB_CUDA(cudaSetDevice(c->device));
     rc = drain(c);
@@ -957,6 +1054,8 @@ int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, u
     const size_t rows = (size_t)h * c->nstreams;
     const size_t bgw = (size_t)w * P.bg_channels;         // bytes per row of img_bgmodel
     uint8_t *d_in = c->d_ring[c->ring_pos];
+    const int fmt = c->input_format;       // YUV: the upload lands in d_yuv and is converted into the ring slot
+    if (fmt != BGSB_INPUT_BGR && (rc = ensure_yuv_staging(c))) return rc;
     const bool out_fg = mask_due(c), want_bg = bg_due(c, bg);
     // FD / WMV: history = the previous upload(s) in the ring -- no copy, the frame is read once
     const bool own_hist = !P.ring_history;
@@ -974,8 +1073,13 @@ int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, u
     auto mark = [&](int i, cudaStream_t st) { if (tracing) cudaEventRecord(c->ev_t[i], st); };
     if (nchunks == 1) {
         mark(0, c->stream);
-        BGSB_CUDA(copy_rows(d_in, (size_t)w * 3, bgr, stride, (size_t)w * 3, rows, cudaMemcpyHostToDevice, c->stream));
+        if (fmt != BGSB_INPUT_BGR) BGSB_CUDA(upload_yuv(fmt, c->d_yuv, bgr, stride, w, h, 0, h, c->nstreams, c->stream));
+        else BGSB_CUDA(copy_rows(d_in, (size_t)w * 3, bgr, stride, (size_t)w * 3, rows, cudaMemcpyHostToDevice, c->stream));
         mark(1, c->stream); mark(2, c->stream);
+        if (fmt != BGSB_INPUT_BGR) {
+            rc = convert_yuv(fmt, c->d_yuv, w, h, 0, h, c->nstreams, d_in, c->stream);
+            if (rc) return rc;
+        }
         if (out_fg || P.warmup_launch) {
             rc = launch_range(c, d_in, 1, c->d_fg, want_bg ? c->d_bg : nullptr, 0, own_hist, c->stream, 0, c->npx);
             if (rc) return rc;
@@ -993,12 +1097,17 @@ int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, u
             const int r0 = i * band, nr = std::min(band, h - r0);
             const size_t p0 = (size_t)r0 * w;
             if (i == 0) mark(0, c->s_h2d);
-            BGSB_CUDA(copy_rows(d_in + p0 * 3, (size_t)w * 3, bgr + (size_t)r0 * stride, stride, (size_t)w * 3, nr,
-                                        cudaMemcpyHostToDevice, c->s_h2d));
+            if (fmt != BGSB_INPUT_BGR) BGSB_CUDA(upload_yuv(fmt, c->d_yuv, bgr, stride, w, h, r0, nr, 1, c->s_h2d));
+            else BGSB_CUDA(copy_rows(d_in + p0 * 3, (size_t)w * 3, bgr + (size_t)r0 * stride, stride, (size_t)w * 3, nr,
+                                     cudaMemcpyHostToDevice, c->s_h2d));
             BGSB_CUDA(cudaEventRecord(c->ev_up[i], c->s_h2d));
             if (i == nchunks - 1) mark(1, c->s_h2d);
             BGSB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_up[i], 0));
             if (i == 0) mark(2, c->stream);
+            if (fmt != BGSB_INPUT_BGR) {       // bands are multiples of 32 rows: whole chroma rows
+                rc = convert_yuv(fmt, c->d_yuv, w, h, r0, nr, 1, d_in, c->stream);
+                if (rc) return rc;
+            }
             rc = launch_range(c, d_in, 1, c->d_fg, want_bg ? c->d_bg : nullptr, 0, own_hist, c->stream, p0, nr * w);
             if (rc) return rc;
             BGSB_CUDA(cudaEventRecord(c->ev_k[i], c->stream));
@@ -1045,7 +1154,7 @@ int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, u
 int bgsb_submit(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, uint8_t *fg, size_t fg_stride,
                 uint8_t *bg, size_t bg_stride, int *fg_valid, int *bg_valid)
 {
-    int rc = check_host_frame(c, bgr, w, stride, fg, fg_stride, bg, bg_stride);
+    int rc = check_host_frame(c, bgr, w, h, stride, fg, fg_stride, bg, bg_stride);
     if (rc) return rc;
     BGSB_CUDA(cudaSetDevice(c->device));
     if (c->w != w || c->h != h) {                                  // geometry change: nothing may be in flight
@@ -1069,12 +1178,19 @@ int bgsb_submit(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, ui
     const bool own_hist = !P.ring_history;
     const int slot = (int)(c->seq & 1);
     uint8_t *o_fg = slot ? c->d_fg2 : c->d_fg, *o_bg = slot ? c->d_bg2 : c->d_bg;
+    const int fmt = c->input_format;
+    if (fmt != BGSB_INPUT_BGR && (rc = ensure_yuv_staging(c))) { drain(c); return rc; }
 
-    // the input buffer (ring slot) was last read by the previous frame's kernel
+    // the input buffer (ring slot, or the YUV staging) was last read by the previous frame's kernels
     if (c->seq > 0) BGSB_CUDA(cudaStreamWaitEvent(c->s_h2d, c->ev_k[slot ^ 1], 0));
-    BGSB_CUDA(copy_rows(d_in, (size_t)w * 3, bgr, stride, (size_t)w * 3, rows, cudaMemcpyHostToDevice, c->s_h2d));
+    if (fmt != BGSB_INPUT_BGR) BGSB_CUDA(upload_yuv(fmt, c->d_yuv, bgr, stride, w, h, 0, h, c->nstreams, c->s_h2d));
+    else BGSB_CUDA(copy_rows(d_in, (size_t)w * 3, bgr, stride, (size_t)w * 3, rows, cudaMemcpyHostToDevice, c->s_h2d));
     BGSB_CUDA(cudaEventRecord(c->ev_up[slot], c->s_h2d));
     BGSB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_up[slot], 0));
+    if (fmt != BGSB_INPUT_BGR) {
+        rc = convert_yuv(fmt, c->d_yuv, w, h, 0, h, c->nstreams, d_in, c->stream);
+        if (rc) return rc;
+    }
     if (out_fg || P.warmup_launch) {
         BGSB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_dn[slot], 0));       // output slot free (no-op until recorded)
         rc = launch_range(c, d_in, 1, o_fg, want_bg ? o_bg : nullptr, 0, own_hist, c->stream, 0, c->npx);
@@ -1107,9 +1223,17 @@ int bgsb_process_fanout(bgsb_ctx *const *ctxs, int n, const uint8_t *bgr, int w,
                         int *fg_valid, int *bg_valid)
 {
     BGSB_REQUIRE(ctxs && bgr && fg && fg_stride && n >= 1 && n <= 16, "bad args");
-    BGSB_REQUIRE(stride >= (size_t)w * 3, "stride smaller than a row");
+    for (int k = 0; k < n; k++) BGSB_REQUIRE(ctxs[k], "null ctx");
     bgsb_ctx *c0 = ctxs[0];
-    for (int k = 0; k < n; k++) { BGSB_REQUIRE(ctxs[k], "null ctx"); if (int drc = drain(ctxs[k])) return drc; }
+    const int fmt = c0->input_format;      // YUV: each band is uploaded once and converted once into the shared frame
+    if (fmt != BGSB_INPUT_BGR) {
+        int rc = check_yuv_frame(fmt, w, h, stride);
+        if (rc) return rc;
+    }
+    BGSB_REQUIRE(stride >= (size_t)w * (fmt == BGSB_INPUT_BGR ? 3 : 1), "stride smaller than a row");
+    for (int k = 0; k < n; k++)
+        BGSB_REQUIRE(ctxs[k]->input_format == fmt, "fan-out contexts must share one \"inputFormat\"");
+    for (int k = 0; k < n; k++) { if (int drc = drain(ctxs[k])) return drc; }
     for (int k = 0; k < n; k++) {
         BGSB_REQUIRE(ctxs[k] && fg[k], "null context or mask buffer");
         BGSB_REQUIRE(ctxs[k]->device == c0->device && ctxs[k]->nstreams == 1, "fan-out takes single-stream contexts of one device");
@@ -1121,6 +1245,10 @@ int bgsb_process_fanout(bgsb_ctx *const *ctxs, int n, const uint8_t *bgr, int w,
     BGSB_CUDA(cudaSetDevice(c0->device));
     for (int k = 0; k < n; k++) {
         int rc = host_setup(ctxs[k], w, h);
+        if (rc) return rc;
+    }
+    if (fmt != BGSB_INPUT_BGR) {
+        int rc = ensure_yuv_staging(c0);
         if (rc) return rc;
     }
     const size_t fbytes = (size_t)w * h * 3;
@@ -1141,8 +1269,14 @@ int bgsb_process_fanout(bgsb_ctx *const *ctxs, int n, const uint8_t *bgr, int w,
     for (int i = 0; i < nchunks; i++) {
         const int r0 = i * band, nr = std::min(band, h - r0);
         const size_t p0 = (size_t)r0 * w;
-        BGSB_CUDA(copy_rows(c0->d_fan + p0 * 3, (size_t)w * 3, bgr + (size_t)r0 * stride, stride, (size_t)w * 3, nr,
-                            cudaMemcpyHostToDevice, c0->s_h2d));
+        if (fmt != BGSB_INPUT_BGR) {
+            BGSB_CUDA(upload_yuv(fmt, c0->d_yuv, bgr, stride, w, h, r0, nr, 1, c0->s_h2d));
+            int rc = convert_yuv(fmt, c0->d_yuv, w, h, r0, nr, 1, c0->d_fan, c0->s_h2d);
+            if (rc) return rc;
+        } else {
+            BGSB_CUDA(copy_rows(c0->d_fan + p0 * 3, (size_t)w * 3, bgr + (size_t)r0 * stride, stride, (size_t)w * 3, nr,
+                                cudaMemcpyHostToDevice, c0->s_h2d));
+        }
         BGSB_CUDA(cudaEventRecord(c0->ev_up[i], c0->s_h2d));
         for (int k = 0; k < n; k++) {
             bgsb_ctx *c = ctxs[k];

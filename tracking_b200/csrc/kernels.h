@@ -191,6 +191,20 @@ struct MorphIO {
 };
 int launch_morph_chain_io(const MorphIO &io, int w, int h, int nimages, const int *ops, int nops, cudaStream_t stream);
 
+// ---- ingest: YUV 4:2:0 to dense BGR, as cv::cvtColor(COLOR_YUV2BGR_NV12 / _I420) (ingest/yuv420.cu) ----
+struct Yuv420Launch {
+    const uint8_t *y;        // first Y row of frame 0
+    const uint8_t *u;        // first chroma row of frame 0: NV12 interleaved U,V; I420 the U plane
+    const uint8_t *v;        // I420: first V row of frame 0 (unused for NV12)
+    size_t y_pitch, c_pitch; // bytes between Y rows / chroma rows
+    size_t src_frame_stride; // bytes between frames (the same for y, u and v)
+    uint8_t *bgr;            // [nframes][rows][w][3], frames dst_frame_stride bytes apart
+    size_t dst_frame_stride;
+    int w, rows, nframes;    // w and rows even: rows / 2 chroma rows per frame
+    int planar;              // 0 NV12, 1 I420
+};
+int launch_yuv420_to_bgr(const Yuv420Launch &L, cudaStream_t stream);
+
 // ---- synthetic video ----------------------------------------------------------------------------
 int launch_synth(uint8_t *d_frames, int nstreams, int T, int w, int h, int t0, uint32_t seed0,
                  cudaStream_t stream);

@@ -72,6 +72,7 @@ struct GpuGroup {
 struct bgsb_pool {
     int algo = 0, nstreams = 0, w = 0, h = 0, ring = 2, table_rows = 256;
     int zero_border = 1;                             // the pipelines' "zeroBorder"
+    int input_format = BGSB_INPUT_BGR;               // "inputFormat": frame_bytes is h*w*3, or h*w*3/2 for YUV 4:2:0
     bool waited[POOL_RING_MAX] = {};                 // the slot's last submit has been waited for
     std::vector<GpuGroup *> groups;
     std::vector<int> group_of, index_in_group;      // per global stream
@@ -206,6 +207,23 @@ static int alloc_tables(bgsb_pool *P)
     return BGSB_OK;
 }
 
+// the frame rings at P->frame_bytes per stream ("inputFormat" before the first submit)
+static int alloc_frames(bgsb_pool *P)
+{
+    for (GpuGroup *G : P->groups) {
+        const size_t bytes = G->streams.size() * P->frame_bytes;
+        BGSB_CUDA(cudaSetDevice(G->device));
+        for (int k = 0; k < P->ring; k++) {
+            if (G->h_in[k]) cudaFreeHost(G->h_in[k]);
+            cudaFree(G->d_in[k]);
+            G->h_in[k] = nullptr; G->d_in[k] = nullptr;
+            BGSB_CUDA(cudaHostAlloc((void **)&G->h_in[k], bytes, cudaHostAllocDefault));
+            BGSB_CUDA(cudaMalloc(&G->d_in[k], bytes));
+        }
+    }
+    return BGSB_OK;
+}
+
 extern "C" {
 
 int bgsb_pool_create(bgsb_pool **out, int algo, int nstreams, const int *devices, int ndevices, int w, int h, int ring)
@@ -274,6 +292,22 @@ int bgsb_pool_set_param(bgsb_pool *P, const char *key, double v)
         BGSB_REQUIRE(v >= 1 && v <= (1 << 24), "tableRows in [1, 2^24]");
         P->table_rows = (int)v;
         return alloc_tables(P);
+    }
+    if (std::string(key) == "inputFormat") {
+        BGSB_REQUIRE(P->seq == 0, "inputFormat: set it before the first submit");
+        BGSB_REQUIRE(v == BGSB_INPUT_BGR || v == BGSB_INPUT_NV12 || v == BGSB_INPUT_I420,
+                     "inputFormat is 0 (BGSB_INPUT_BGR), 1 (BGSB_INPUT_NV12) or 2 (BGSB_INPUT_I420)");
+        BGSB_REQUIRE(v == BGSB_INPUT_BGR || (P->w % 2 == 0 && P->h % 2 == 0),
+                     "YUV 4:2:0 input (inputFormat NV12 / I420) needs an even width and height");
+        for (GpuGroup *G : P->groups) {
+            int rc = bgsb_pipeline_set_param(G->pipe, key, v);
+            if (rc) return rc;
+        }
+        P->input_format = (int)v;
+        const size_t npx = (size_t)P->w * P->h, fb = v == BGSB_INPUT_BGR ? npx * 3 : npx * 3 / 2;
+        if (fb == P->frame_bytes) return BGSB_OK;
+        P->frame_bytes = fb;
+        return alloc_frames(P);
     }
     for (GpuGroup *G : P->groups) {
         int rc = bgsb_pipeline_set_param(G->pipe, key, v);

@@ -64,6 +64,7 @@ class StreamPool:
             capi.check(L.bgsb_pool_set_morph(self._h, ops, n))
         for k, v in params.items():
             capi.check(L.bgsb_pool_set_param(self._h, k.encode(), float(v)))
+        self.input_format = int(params.get("inputFormat", capi.INPUT_BGR))
         rows = C.c_int(0)
         capi.check(L.bgsb_pool_info(self._h, None, None, C.byref(rows)))
         self.table_rows = rows.value
@@ -85,12 +86,14 @@ class StreamPool:
         return d.value
 
     def frame_buffer(self, stream, slot):
-        """(h, w, 3) uint8 view of the page-locked buffer the capture side fills for (stream, slot)."""
+        """(h, w, 3) uint8 view of the page-locked buffer the capture side fills for (stream, slot); with "inputFormat"
+        NV12 / I420 the (3h/2, w) view of the YUV 4:2:0 image."""
         p = capi.lib().bgsb_pool_frame_buffer(self._h, stream, slot)
         if not p:
             raise IndexError("stream / slot out of range")
-        buf = (C.c_uint8 * (self.h * self.w * 3)).from_address(p)
-        return np.frombuffer(buf, dtype=np.uint8).reshape(self.h, self.w, 3)
+        shape = (self.h, self.w, 3) if self.input_format == capi.INPUT_BGR else (self.h * 3 // 2, self.w)
+        buf = (C.c_uint8 * int(np.prod(shape))).from_address(p)
+        return np.frombuffer(buf, dtype=np.uint8).reshape(shape)
 
     def submit(self, slot, want_masks=False, detect=False):
         """want_masks: download the cleaned masks (mask()); detect: keep them on the device for detect()."""
