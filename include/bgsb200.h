@@ -130,8 +130,7 @@ BGSB_API int bgsb_reset(bgsb_ctx *ctx);
  * "complexityReductionThreshold" 0.05, "detectShadows" 1, "shadowValue" 127,
  * "shadowThreshold" 0.5 (varMin / varMax given in the wrong order are swapped, as OpenCV does); and "grayVariant": 0 = OpenCV 4.x BGR2GRAY constants, 1 = 2.4.x;
  * "kernelVariant" (MOG2): 0 = production kernels, 1 = straight restatement kernel (identical results, kept for
- * A/B measurements).  (8, 9 = timing instruments with WRONG results exist only in a library built with
- * -DBGSB_INSTRUMENT for tools/floor_probe.py; the shipped library rejects them);
+ * A/B measurements; any other value is refused);
  * "ablTable" (AdaptiveBackgroundLearning): 1 = lookup-table kernels (default), 2 = only the per-thread table kernel,
  * 3 = as 1, with the bulk-copy kernel whenever the geometry allows (by default only for groups of ~3.6 Mpx and more),
  * 0 = arithmetic kernel -- identical results;

@@ -12,15 +12,12 @@ bit-exact, so a parity test alone cannot tell which one it checked.  Each row be
      names to equal the row's expected set (for a routing boundary this is the fallback form, so the fast form must
      not run).
 
-The A/B environment switches are read once per process, so their rows run in child processes.  The CPU-only
-inventory check requires every __global__ kernel of tracking_b200/csrc to be the expected kernel of some row.
+The CPU-only inventory check requires every __global__ kernel of tracking_b200/csrc to be the expected kernel of some row.
 """
 import collections
 import glob
 import os
 import re
-import subprocess
-import sys
 import warnings
 
 import numpy as np
@@ -513,62 +510,15 @@ def test_host_call_into_padded_rois(oracle, aid):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# A/B switches: read once per process, so each environment runs its rows in a child process
-
-CHILD_ENV = {
-    "two_pass_stream_no_pdl": {"BGSB_ASBL_TWO_PASS": "1", "BGSB_MOG2_STREAM": "2", "BGSB_NO_PDL": "1"},
-    "per_thread_baselines": {"BGSB_WMV_BULK": "0", "BGSB_WMM_BULK": "0", "BGSB_ABL_BULK": "0", "BGSB_BYTEWISE_COALESCED": "0",
-                             "BGSB_ASBL_QUADS": "0"},
-}
-CHILD_ROWS = {
-    "two_pass_stream_no_pdl": [
-        Row("asbl_quads_two_pass", ASBL, {"asbl_diff4_kernel", "asbl_update4_kernel"}, h=48, w=64, kw=dict(learningFrames=2)),
-        Row("asbl_quads_two_pass_S3_w68", ASBL, {"asbl_diff4_kernel", "asbl_update4_kernel"}, h=48, w=68, S=3,
-            kw=dict(learningFrames=2)),
-        Row("mog2_stream_byte_mask_group", MOG2, {"mog2_t1_stream_kernel"}, h=64, w=64, S=2, skip=1),
-        Row("fd_coalesced_no_pdl", FD, {"fd_coalesced_kernel"}, skip=1),
-    ],
-    "per_thread_baselines": [
-        Row("wmv_bulk_off", WMV, {"wmv_kernel"}),
-        Row("wmm_bulk_off", WMM, {"wmm_kernel"}),
-        Row("abl_bulk_off_table3", ABL, {"abl_lut_coalesced_kernel"}, kw=dict(ablTable=3)),
-        Row("sd_coalesced_off", SD, {"sigma_delta_kernel"}, bg=False, skip=1),
-        Row("amed_coalesced_off", AMED, {"dps_median_kernel"}, bg=False, kw=dict(samplingRate=2), skip=1),
-        Row("asbl_quads_off", ASBL, {"asbl_fused_kernel"}, h=48, w=64, kw=dict(learningFrames=2)),
-    ],
-}
-
-
-def child_main(which):
-    """Entry point of the child process: every row of CHILD_ROWS[which]; an assertion ends it with a nonzero code."""
-    from oracle import restate
-    restate.build()
-    for r in CHILD_ROWS[which]:
-        run_row(restate, r)
-        print("ok", r.id, flush=True)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("which", sorted(CHILD_ENV))
-def test_ab_switch_routes_in_child_process(which):
-    env = dict(os.environ, **CHILD_ENV[which])
-    code = ("import sys; sys.path[:0] = [%r, %r]; import test_gpu_kernel_routes as m; m.child_main(%r)"
-            % (ROOT, os.path.join(ROOT, "tests"), which))
-    res = subprocess.run([sys.executable, "-c", code], env=env, cwd=ROOT, capture_output=True, text=True, timeout=900)
-    assert res.returncode == 0, res.stdout[-3000:] + res.stderr[-6000:]
-    assert res.stdout.count("ok ") == len(CHILD_ROWS[which]), res.stdout
-
-
-# ---------------------------------------------------------------------------------------------------------------------
 # CPU: every kernel of the library has a routed parity row
 
 
 
 def test_every_kernel_has_a_routed_parity_row():
     kernels = library_kernels()
-    assert len(kernels) >= 45
+    assert len(kernels) >= 43
     covered = PIPE_STREAM | PIPE_GROUP | PIPE_PHASES | MORPH_CCL | MOMENTS
-    for r in ROWS + [r for rows in CHILD_ROWS.values() for r in rows]:
+    for r in ROWS:
         covered |= r.expect
     assert covered <= kernels, "rows expect kernels that do not exist: %s" % sorted(covered - kernels)
     for name, test in EXEMPT.items():

@@ -148,7 +148,7 @@ def test_errors_leave_the_context_usable(oracle):
     with pytest.raises(tb.BgsbError):
         p.set("noSuchKey", 1)
     with pytest.raises(tb.BgsbError):
-        p.set("kernelVariant", 9)                # timing instruments are not in the shipped library
+        p.set("kernelVariant", 9)                # kernelVariant is 0 or 1
     assert b"kernelVariant" in L.bgsb_last_error()
     assert p.frame_count == 1
     for x in f[1:]:

@@ -1,5 +1,5 @@
 """ABL: lookup-table kernels vs arithmetic kernel, 1 and 16 streams of 1080p (GPU box, measurement tooling).
-BGSB_ABL_BULK=0 in the environment keeps the register-prefetch kernel instead of the bulk-copy kernel for table=1 (tables 2 and 0 are the per-thread table kernel and the arithmetic kernel)."""
+Table 1 is the production routing, 2 the per-thread table kernel, 0 the arithmetic kernel; --table1 runs table 1 only."""
 import os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -27,6 +27,5 @@ for S in (1, 16):
         dt = e0.elapsed_time(e1) / n * 1e-3
         sig = (int(fg.long().sum()), int(bg.long().sum()))
         if ref is None: ref = sig
-        print("BGSB_ABL_BULK=%s" % os.environ.get("BGSB_ABL_BULK", "-"), end=" ")
         print("S=%d table=%d  %.1f us/step  %.0f GB/s (10 B/px)  same_result=%s" % (S, table, dt * 1e6, S * w * h * 10 / dt / 1e9, sig == ref))
         p.close()

@@ -23,4 +23,4 @@ for k in range(n):
     p.process_dev(d[k % NF].data_ptr(), W, H, fg.data_ptr(), bg.data_ptr(), stream=st)
 e1.record(); torch.cuda.synchronize()
 us = e0.elapsed_time(e1) / n * 1e3
-print(json.dumps(dict(streams=S, geometry=[W, H], stream_form=os.environ.get("BGSB_MOG2_STREAM", "1"), us_per_frame_set=us, us_per_frame_stream=us / S, gpx_s=S * W * H / us / 1e3)))
+print(json.dumps(dict(streams=S, geometry=[W, H], us_per_frame_set=us, us_per_frame_stream=us / S, gpx_s=S * W * H / us / 1e3)))

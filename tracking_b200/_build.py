@@ -1,6 +1,6 @@
 """In-tree build of libbgsb200.so with nvcc for sm_100a (no torch, no JIT cache).
 
-    python -m tracking_b200._build [--force] [--instrument]
+    python -m tracking_b200._build [--force]
 
 The shared library is written next to this file so that it travels to the GPU box with the
 repository snapshot.  Model kernels need OpenCV's unfused fp32 arithmetic, so the whole library
@@ -42,10 +42,8 @@ def needs_build():
     return any(os.path.getmtime(p) > t for p in _deps())
 
 
-def build(force=False, verbose=False, instrument=False):
-    """instrument=True adds -DBGSB_INSTRUMENT: the wrong-result timing modes of the MOG2 kernel (kernelVariant 8 / 9,
-    tools/floor_probe.py).  Never ship such a build."""
-    if not force and not instrument and not needs_build():
+def build(force=False, verbose=False):
+    if not force and not needs_build():
         return LIB
     os.makedirs(OBJDIR, exist_ok=True)
     srcs = [s for s in SOURCES if os.path.exists(os.path.join(CSRC, s))]
@@ -53,11 +51,9 @@ def build(force=False, verbose=False, instrument=False):
     for f in os.listdir(OBJDIR):                 # objects of sources that no longer exist must not travel to the GPU box
         if f not in keep:
             os.remove(os.path.join(OBJDIR, f))
-    flags = FLAGS + (["-DBGSB_INSTRUMENT"] if instrument else [])
-
     def cc(src):
         obj = os.path.join(OBJDIR, _obj_name(src))
-        cmd = [NVCC, *flags, "-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = [NVCC, *FLAGS, "-c", os.path.join(CSRC, src), "-o", obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("nvcc failed for %s:\n%s\n%s" % (src, r.stdout, r.stderr))
@@ -78,4 +74,4 @@ def build(force=False, verbose=False, instrument=False):
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv, instrument="--instrument" in sys.argv))
+    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))

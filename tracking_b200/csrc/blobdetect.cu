@@ -12,7 +12,6 @@
 //   5    drop small blobs and blobs overlapping tracked ones
 //   6    insertion sort by w*h (descending), keep 10
 //   7    track lists over the last `Latency` frames, uniform-motion test, emit best new blob
-#include <chrono>
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -332,17 +331,10 @@ static int detect_impl(bgsb_blobdetector *bd, const uint8_t *d_mask, int w, int 
                        int n_old, bgsb_blob *new_blobs, int new_cap, int *n_new, int *result,
                        bgsb_blob *frame_blobs, int frame_cap, int *n_frame, cudaStream_t stream)
 {
-    static const bool trace = getenv("BGSB_TRACE_DETECT") != nullptr;     // stage times on stderr (debugging aid)
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    auto us = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
-        return std::chrono::duration<double, std::micro>(b - a).count();
-    };
-    const auto t0 = now();
     int rc = ensure_ccl(bd, w, h);
     if (rc) return rc;
     rc = bgsb_ccl_label_dev(bd->ccl, d_mask, w, h, bd->zero_border, nullptr, stream);
     if (rc) return rc;
-    const auto t1 = now();
     int ncomp = 0;
     if (bd->comps.size() < 2048) bd->comps.resize(2048);     // one round trip in the common case
     rc = bgsb_ccl_components(bd->ccl, bd->comps.data(), (int)bd->comps.size(), &ncomp);
@@ -351,19 +343,14 @@ static int detect_impl(bgsb_blobdetector *bd, const uint8_t *d_mask, int w, int 
         rc = bgsb_ccl_components(bd->ccl, bd->comps.data(), (int)bd->comps.size(), &ncomp);
     }
     if (rc) return rc;
-    const auto t2 = now();
     std::vector<int32_t> qrects;
     detect_rects(bd, bd->comps.data(), ncomp, w, h, qrects);
     const int nq = (int)qrects.size() / 4;
-    const auto t3 = now();
     std::vector<uint64_t> mom(6 * (size_t)nq + 6);
     if (nq) {
         rc = bgsb_ccl_rect_moments(bd->ccl, qrects.data(), nq, mom.data());
         if (rc) return rc;
     }
-    if (trace)
-        fprintf(stderr, "detect: launch %.0f us, components(%d) %.0f us, clustering(%d rects) %.0f us, moments %.0f us\n",
-                us(t0, t1), ncomp, us(t1, t2), nq, us(t2, t3), us(t3, now()));
     detect_finish(bd, qrects.data(), nq, mom.data(), w, h, old_blobs, n_old, new_blobs, new_cap, n_new, result, frame_blobs,
                   frame_cap, n_frame);
     return BGSB_OK;

@@ -126,7 +126,7 @@ struct bgsb_ctx {
     size_t prati_bytes = 0;
     int abl_table = 1;         // ABL: 1 = lookup-table kernel, 0 = arithmetic kernel (A/B, identical results)
     int abl_blend = 0, lut_blend = 0;   // ABL: 0 = OpenCV 4.x fp64 addWeighted, 1 = OpenCV 2.4 fp32 addWeighted (table kernels only)
-    int mog2_variant = 0;      // see launch_mog2 (mog2.cu): 0 production, 1 straight restatement, 8/9 timing instruments
+    int mog2_variant = 0;      // see launch_mog2 (mog2.cu): 0 production, 1 straight restatement
     // geometry / counters
     int w = 0, h = 0, npx = 0;
     size_t pstride = 0;
@@ -663,12 +663,6 @@ int sm_count(int device)
     }
     return v;
 }
-
-bool pdl_enabled()
-{
-    static const bool on = [] { const char *e = getenv("BGSB_NO_PDL"); return !(e && e[0] == '1'); }();
-    return on;
-}
 }  // namespace bgsb
 
 // copy streams and per-band events of the upload / kernel / download pipelines
@@ -869,11 +863,7 @@ int bgsb_set_param(bgsb_ctx *c, const char *key, double v)
     }
     else if (k == "quietGroups") c->wmv_quiet = (v != 0);
     else if (k == "trace") c->trace = (v != 0);
-#ifdef BGSB_INSTRUMENT
-    else if (k == "kernelVariant") { BGSB_REQUIRE(v == 0 || v == 1 || v == 8 || v == 9, "kernelVariant is 0 or 1 (8, 9: timing instruments)"); c->mog2_variant = (int)v; }
-#else
     else if (k == "kernelVariant") { BGSB_REQUIRE(v == 0 || v == 1, "kernelVariant is 0 or 1"); c->mog2_variant = (int)v; }
-#endif
     else if (k == "ablTable") {
         BGSB_REQUIRE(v == 0 || v == 1 || v == 2 || v == 3, "ablTable is 0, 1, 2 or 3");
         BGSB_REQUIRE(v != 0 || c->abl_blend == 0, "the OpenCV 2.4 blend (ablBlend 1) exists in table form only");
@@ -1059,9 +1049,7 @@ int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, u
     const bool out_fg = mask_due(c), want_bg = bg_due(c, bg);
     // FD / WMV: history = the previous upload(s) in the ring -- no copy, the frame is read once
     const bool own_hist = !P.ring_history;
-    // BGSB_HOST_BANDS=n: the default band count of contexts that did not set "hostBands" (A/B across processes, e.g. under torchrun)
-    static const int env_bands = [] { const char *e = getenv("BGSB_HOST_BANDS"); const int v = e ? atoi(e) : 0; return (v >= 1 && v <= 8) ? v : 0; }();
-    const int host_bands = c->host_bands_auto ? (env_bands ? env_bands : (want_bg ? 3 : 2)) : c->host_bands;
+    const int host_bands = c->host_bands_auto ? (want_bg ? 3 : 2) : c->host_bands;
     const Bands B = plan_bands(w, h, (c->nstreams == 1 && out_fg && !P.stencil) ? host_bands : 1);
     const int nchunks = B.n, band = B.rows;
     // stage timing (parameter "trace" or BGSB_TRACE=1): events around the uploads, the kernels and the downloads
@@ -1373,33 +1361,21 @@ int bgsb_copy_probe(int device, size_t bytes_up, size_t bytes_down, int iters, d
     BGSB_REQUIRE(bytes_up > 0 && bytes_down > 0 && iters >= 1 && sec_up && sec_down && sec_both, "bad args");
     BGSB_CUDA(cudaSetDevice(device));
     void *h_up = nullptr, *h_dn = nullptr, *d_up = nullptr, *d_dn = nullptr;
-    // BGSB_PROBE_WC=1: the upload buffer as write-combined memory (what bgsb_host_alloc(.., 1) hands out for input frames)
-    static const bool wc = [] { const char *e = getenv("BGSB_PROBE_WC"); return e && e[0] == '1'; }();
-    // BGSB_PROBE_SPLIT=k (1..4): each transfer as k pieces on k streams (k copy engines per direction)
-    static const int nsplit = [] { const char *e = getenv("BGSB_PROBE_SPLIT"); int k = e ? atoi(e) : 1; return k < 1 ? 1 : (k > 4 ? 4 : k); }();
-    cudaStream_t su[4] = {nullptr, nullptr, nullptr, nullptr}, sd[4] = {nullptr, nullptr, nullptr, nullptr};
-    cudaError_t e = cudaHostAlloc(&h_up, bytes_up, wc ? cudaHostAllocWriteCombined : cudaHostAllocDefault);
+    cudaStream_t su = nullptr, sd = nullptr;
+    cudaError_t e = cudaHostAlloc(&h_up, bytes_up, cudaHostAllocDefault);
     if (e == cudaSuccess) e = cudaHostAlloc(&h_dn, bytes_down, cudaHostAllocDefault);
     if (e == cudaSuccess) e = cudaMalloc(&d_up, bytes_up);
     if (e == cudaSuccess) e = cudaMalloc(&d_dn, bytes_down);
-    for (int i = 0; i < nsplit && e == cudaSuccess; i++) {
-        e = cudaStreamCreateWithFlags(&su[i], cudaStreamNonBlocking);
-        if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&sd[i], cudaStreamNonBlocking);
-    }
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&su, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&sd, cudaStreamNonBlocking);
     if (e == cudaSuccess) { memset(h_up, 1, bytes_up); memset(h_dn, 0, bytes_down); }
-    auto piece = [&](size_t bytes, int i, size_t *off) { const size_t per = (bytes / nsplit) & ~(size_t)255; *off = per * i; return i == nsplit - 1 ? bytes - per * i : per; };
     auto issue = [&](bool up, bool down) {
-        for (int i = 0; i < nsplit && e == cudaSuccess; i++) {
-            size_t off = 0, n = 0;
-            if (up) { n = piece(bytes_up, i, &off); e = cudaMemcpyAsync((char *)d_up + off, (char *)h_up + off, n, cudaMemcpyHostToDevice, su[i]); }
-            if (down && e == cudaSuccess) { n = piece(bytes_down, i, &off); e = cudaMemcpyAsync((char *)h_dn + off, (char *)d_dn + off, n, cudaMemcpyDeviceToHost, sd[i]); }
-        }
+        if (up && e == cudaSuccess) e = cudaMemcpyAsync(d_up, h_up, bytes_up, cudaMemcpyHostToDevice, su);
+        if (down && e == cudaSuccess) e = cudaMemcpyAsync(h_dn, d_dn, bytes_down, cudaMemcpyDeviceToHost, sd);
     };
     auto sync_all = [&]() {
-        for (int i = 0; i < nsplit; i++) {
-            if (e == cudaSuccess) e = cudaStreamSynchronize(su[i]);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(sd[i]);
-        }
+        if (e == cudaSuccess) e = cudaStreamSynchronize(su);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(sd);
     };
     auto run = [&](bool up, bool down) -> double {
         for (int w = 0; w < 3; w++) issue(up, down);
@@ -1412,7 +1388,8 @@ int bgsb_copy_probe(int device, size_t bytes_up, size_t bytes_down, int iters, d
     if (e == cudaSuccess) *sec_up = run(true, false);
     if (e == cudaSuccess) *sec_down = run(false, true);
     if (e == cudaSuccess) *sec_both = run(true, true);
-    for (int i = 0; i < 4; i++) { if (su[i]) cudaStreamDestroy(su[i]); if (sd[i]) cudaStreamDestroy(sd[i]); }
+    if (su) cudaStreamDestroy(su);
+    if (sd) cudaStreamDestroy(sd);
     cudaFree(d_up); cudaFree(d_dn);
     if (h_up) cudaFreeHost(h_up);
     if (h_dn) cudaFreeHost(h_dn);

@@ -57,8 +57,6 @@ __device__ __forceinline__ void pdl_entry()
     asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
-bool pdl_enabled();     // capi.cu
-
 template <typename... KArgs, typename... Args>
 inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args &&... args)
 {
@@ -67,7 +65,7 @@ inline void launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 1 : 0;          // BGSB_NO_PDL=1: plain stream order (A/B)
+    cfg.attrs = attr; cfg.numAttrs = 1;
     const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
     if (e != cudaSuccess && g_launch_status == cudaSuccess) g_launch_status = e;     // reported by BGSB_LAUNCH_CHECK
 }

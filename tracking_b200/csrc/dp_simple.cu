@@ -526,11 +526,10 @@ dps_median_coalesced_kernel(DpsLaunch L)
     st_stream_u4(L.fg + s * L.fg_stride + (size_t)chunk * BW_CHUNK_PX + lane * 16u, mask);
 }
 
-// whole chunks, 16-byte aligned images and strides; BGSB_BYTEWISE_COALESCED=0 keeps the 4-pixel kernels (A/B)
+// whole chunks, 16-byte aligned images and strides
 static bool bw_coalesced_ok(int npx, int nstreams, std::initializer_list<const void *> ptrs, std::initializer_list<size_t> strides)
 {
-    static const bool off = [] { const char *e = getenv("BGSB_BYTEWISE_COALESCED"); return e && e[0] == '0'; }();
-    if (off || npx < BW_CHUNK_PX || npx % BW_CHUNK_PX) return false;
+    if (npx < BW_CHUNK_PX || npx % BW_CHUNK_PX) return false;
     for (const void *p : ptrs) if (reinterpret_cast<uintptr_t>(p) & 15) return false;
     if (nstreams > 1) for (size_t st : strides) if (st & 15) return false;
     return true;

@@ -51,7 +51,7 @@ struct AsblLaunch {
     int first;               // no model yet: it starts as the gray input (AdaptiveSelectiveBackgroundLearning.cpp:47-48)
     int selective;           // 0: learning phase, every pixel is blended (:65-71); 1: only background pixels (:72-90)
     double alpha;            // alphaLearn or alphaDetection
-    const uint8_t *lut;      // 64 KB blend table for alpha (launch_abl_lut_build), nullable: blend in arithmetic
+    const uint8_t *lut;      // 64 KB blend table for alpha (launch_abl_lut_build): the single-pass kernels blend through it
     int thr, gray_variant;
 };
 // *swapped = 1: the new model is in model_out (the caller exchanges the two buffers), 0: updated in place

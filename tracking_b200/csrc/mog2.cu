@@ -144,18 +144,14 @@ mog2_kernel(const __grid_constant__ Mog2Launch L)
     st_stream_u32(nmp, (unsigned)n[0] | ((unsigned)n[1] << 8) | ((unsigned)n[2] << 16) | ((unsigned)n[3] << 24));
 }
 
-int launch_mog2_t1(const Mog2Launch &L, int nstreams, int mode, cudaStream_t stream);
+int launch_mog2_t1(const Mog2Launch &L, int nstreams, cudaStream_t stream);
 int launch_mog2_fused(const Mog2Launch &L, int nstreams, cudaStream_t stream);
 
 // variant: 0 production (T == 1: two-phase kernel; T > 1: temporal-fusion kernel; csrc/mog2_t1.cu)
 //          1 straight restatement (this file) -- the reference point of profiles/r1_mog2_kernel_history.md
-//          8, 9 (-DBGSB_INSTRUMENT builds only) timing instruments with wrong results: T == 1 kernel without its
-//          generic phase / without arithmetic
 int launch_mog2(const Mog2Launch &L, int nstreams, int variant, cudaStream_t stream)
 {
-    if (variant == 0) return L.T == 1 ? launch_mog2_t1(L, nstreams, 0, stream) : launch_mog2_fused(L, nstreams, stream);
-    if (variant == 9) return launch_mog2_t1(L, nstreams, 1, stream);
-    if (variant == 8) return launch_mog2_t1(L, nstreams, 2, stream);
+    if (variant == 0) return L.T == 1 ? launch_mog2_t1(L, nstreams, stream) : launch_mog2_fused(L, nstreams, stream);
     const int threads = 128;
     long long nthreads = ((long long)L.npx + PX - 1) / PX;
     dim3 grid((unsigned)((nthreads + threads - 1) / threads), (unsigned)nstreams);
