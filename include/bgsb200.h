@@ -235,7 +235,8 @@ BGSB_API int bgsb_frame_count(bgsb_ctx *ctx, int64_t *nframes);
 /* Bytes of HBM model state held per stream (101 B/px for MOG2). */
 BGSB_API int bgsb_state_bytes(bgsb_ctx *ctx, size_t *bytes);
 /* Raw MOG2 state export/import (SURVEY 8f N4): K planes each of weight, variance,
- * mean B, G, R as fp32 [25][npx] followed by nmodes u8 [npx]; host buffers. */
+ * mean B, G, R as fp32 [25][npx] followed by nmodes u8 [npx]; host buffers.
+ * Import refuses a mode count above 5 (BGSB_ERR_ARG) and then leaves the context as it was. */
 BGSB_API int bgsb_mog2_export_state(bgsb_ctx *ctx, int stream_index, float *planes, uint8_t *nmodes);
 BGSB_API int bgsb_mog2_import_state(bgsb_ctx *ctx, int stream_index, int w, int h, int64_t nframes,
                                     const float *planes, const uint8_t *nmodes);

@@ -1331,6 +1331,10 @@ int bgsb_mog2_import_state(bgsb_ctx *c, int si, int w, int h, int64_t nframes, c
     BGSB_REQUIRE(c->algo == BGSB_ALGO_MOG2, "not a MOG2 context");
     BGSB_REQUIRE(si >= 0 && si < c->nstreams, "stream index");
     BGSB_REQUIRE(nframes >= 1, "nframes >= 1");
+    BGSB_REQUIRE(w > 0 && h > 0, "empty frame");
+    // a mode count above K would make the kernels walk past the pixel's K modes: refused before anything changes
+    for (size_t i = 0, n = (size_t)w * h; i < n; i++)
+        BGSB_REQUIRE(nmodes[i] <= MOG2_K, "nmodes above 5");
     BGSB_CUDA(cudaSetDevice(c->device));
     int rc = ensure_geometry(c, w, h);
     if (rc) return rc;
