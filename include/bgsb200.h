@@ -157,7 +157,17 @@ BGSB_API int bgsb_reset(bgsb_ctx *ctx);
  * the BGR upload would fill; the device paths convert into a library-owned scratch on the caller's stream first.  The
  * model and the history are kept as BGR, so the format may change between calls.  BGSB_ERR_ARG for an odd w or h, an
  * I420 host frame with stride != w, and together with "retainInput" (the converted frames are the library's, so the
- * caller's buffers cannot serve as the history).  Fan-out contexts must share one format. */
+ * caller's buffers cannot serve as the history).  Fan-out contexts must share one format;
+ * "gaussianBlur" (0 or 1, default 0): the reference PreProcessor's gaussianBlur switch (FrameProcessor.cpp:173-174).  1 =
+ * every frame is blurred on the device, exactly as cv::GaussianBlur(img, Size(7, 7), 1.5) does on 8-bit BGR (OpenCV 4.x,
+ * BORDER_REFLECT_101), before the plugin sees it: on every entry point, after the YUV conversion with a YUV
+ * "inputFormat", and on warm-up frames too, so the history FrameDifference / WeightedMovingVariance / WeightedMovingMean
+ * keep is the blurred frame.  A change takes effect from the next frame.  The host paths upload into a staging buffer
+ * and blur into the buffer the upload would fill; the device paths blur into a library-owned scratch on the caller's
+ * stream.  BGSB_ERR_ARG for any other value, and together with "retainInput" in either order (the history is the
+ * blurred frame, so the caller's buffers cannot serve as it).  Fan-out contexts must share one value.  A C++ caller that
+ * keeps FrameProcessor's PreProcessor with only gaussianBlur enabled sets this key on each GPU plugin and hands them
+ * img_input instead of img_prep (INTEGRATION.md 4b). */
 BGSB_API int bgsb_set_param(bgsb_ctx *ctx, const char *key, double value);
 BGSB_API int bgsb_get_param(bgsb_ctx *ctx, const char *key, double *value);
 

@@ -18,7 +18,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJDIR = os.path.join(HERE, "_obj")
 LIB = os.path.join(HERE, "libbgsb200.so")
 SOURCES = ["capi.cu", "simple_bgs.cu", "mog2.cu", "mog2_t1.cu", "dpz.cu", "dp_simple.cu", "synth.cu", "morph.cu", "ccl.cu", "blobdetect.cu", "pipeline.cu", "pool.cu",
-           os.path.join("ingest", "yuv420.cu")]
+           os.path.join("ingest", "yuv420.cu"), os.path.join("prep", "gauss7.cu")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-fmad=false",
          "-Xcompiler", "-fPIC,-fvisibility=hidden", "-Xptxas", "-v"]

@@ -95,7 +95,8 @@ class _Plugin:
     # -- IBGS::process, host buffers -------------------------------------------------------
     def process(self, img_input, want_bg=True):
         """img_input: HxWx3 uint8 BGR (a group takes nstreams x H x W x 3); with "inputFormat" NV12 / I420 the
-        (3h/2) x W YUV image (a group: nstreams x 3h/2 x W).  Returns (img_output | None, img_bgmodel | None)."""
+        (3h/2) x W YUV image (a group: nstreams x 3h/2 x W).  With "gaussianBlur" 1 the plugin sees the frame as
+        cv::GaussianBlur(img, Size(7, 7), 1.5) gives it, blurred on the device.  Returns (img_output | None, img_bgmodel | None)."""
         if img_input is None or img_input.size == 0:      # `if(img_input.empty()) return;`
             return None, None
         if self.input_format != capi.INPUT_BGR:
@@ -306,7 +307,8 @@ def pinned_empty(shape, write_combined=False):
 def process_fanout(plugins, img_input, want_bg=True):
     """FrameProcessor::process (FrameProcessor.cpp:169-215): every plugin on the same frame, one upload.
     Returns [(img_output | None, img_bgmodel | None), ...] exactly as plugin.process(img_input) would for each.
-    With "inputFormat" NV12 / I420 (the same on every plugin) img_input is the (3h/2) x W YUV image."""
+    With "inputFormat" NV12 / I420 (the same on every plugin) img_input is the (3h/2) x W YUV image.  With "gaussianBlur"
+    1 (the same on every plugin) the frame is blurred once on the device and every plugin sees the blurred frame."""
     if img_input is None or img_input.size == 0:
         return [(None, None) for _ in plugins]
     fmt = plugins[0].input_format if plugins else capi.INPUT_BGR

@@ -167,6 +167,12 @@ struct bgsb_ctx {
     uint8_t *d_yuv = nullptr;             // host paths: the uploaded YUV frames [S][3h/2][w] (fan-out: the first context's)
     uint8_t *d_conv = nullptr;            // device paths: the converted frames [S][T][h][w][3]
     size_t d_conv_bytes = 0;
+    // "gaussianBlur": the reference PreProcessor's cv::GaussianBlur(Size(7, 7), 1.5), which prep/gauss7.cu applies to
+    // every BGR frame (after the YUV conversion) before the plugin sees it; the history is the blurred frame
+    int gaussian_blur = 0;
+    uint8_t *d_prep = nullptr;            // host paths: the BGR frames before the blur [S][h][w][3] (fan-out: the first context's)
+    uint8_t *d_blur = nullptr;            // device paths: the blurred frames [S][T][h][w][3]
+    size_t d_blur_bytes = 0;
     // WMV quiet-group shortcut: wmv_bound[ew][r] = largest standard-deviation byte over all triples of range r for the
     // weight set ew (computed once per weight set on the device, launch_wmv_bound_table); wmv_quiet 0 switches it off
     int wmv_quiet = 1;
@@ -193,6 +199,7 @@ static void free_staging(bgsb_ctx *c)
     cudaFree(c->d_fg2); c->d_fg2 = nullptr;
     cudaFree(c->d_bg2); c->d_bg2 = nullptr;
     cudaFree(c->d_yuv); c->d_yuv = nullptr;
+    cudaFree(c->d_prep); c->d_prep = nullptr;
 }
 
 static void free_buffers(bgsb_ctx *c)
@@ -204,6 +211,7 @@ static void free_buffers(bgsb_ctx *c)
     free_staging(c);
     cudaFree(c->d_fan); c->d_fan = nullptr; c->d_fan_bytes = 0;
     cudaFree(c->d_conv); c->d_conv = nullptr; c->d_conv_bytes = 0;
+    cudaFree(c->d_blur); c->d_blur = nullptr; c->d_blur_bytes = 0;
     cudaFree(c->d_prati); c->d_prati = nullptr; c->prati_bytes = 0; c->prati_n = c->prati_pos = 0;
     c->w = c->h = c->npx = 0; c->pstride = 0;
     c->nframes = 0; c->mog2_epoch = 0; c->have_hist = 0; c->ring_pos = 0;
@@ -337,6 +345,27 @@ static int ensure_yuv_staging(bgsb_ctx *c)
 {
     if (c->d_yuv) return BGSB_OK;
     const cudaError_t e = cudaMalloc(&c->d_yuv, (size_t)c->nstreams * c->npx * 3 / 2);
+    if (e != cudaSuccess) return staging_fail(c, e);
+    return BGSB_OK;
+}
+
+// ---- "gaussianBlur" --------------------------------------------------------------------------------
+// Output rows [r0, r0 + nr) of `nframes` dense BGR frames at src -> the same rows at dst.  Rows up to 3 beyond the band
+// are read, so on the host paths band i is blurred only once band i + 1 has arrived.
+static int blur_frames(const uint8_t *src, int w, int h, int r0, int nr, int nframes, uint8_t *dst, cudaStream_t st)
+{
+    Gauss7Launch L;
+    memset(&L, 0, sizeof(L));
+    L.src = src; L.dst = dst; L.frame_stride = (size_t)w * h * 3;
+    L.w = w; L.h = h; L.r0 = r0; L.nr = nr; L.nframes = nframes;
+    return launch_gauss7(L, st);
+}
+
+// host paths with the blur: the uploaded (or converted) BGR frames land here and are blurred into the ring slot
+static int ensure_prep_staging(bgsb_ctx *c)
+{
+    if (c->d_prep) return BGSB_OK;
+    const cudaError_t e = cudaMalloc(&c->d_prep, (size_t)c->nstreams * c->npx * 3);
     if (e != cudaSuccess) return staging_fail(c, e);
     return BGSB_OK;
 }
@@ -852,7 +881,15 @@ int bgsb_set_param(bgsb_ctx *c, const char *key, double v)
     else if (k == "retainInput") {
         BGSB_REQUIRE(v == 0 || c->input_format == BGSB_INPUT_BGR, "retainInput cannot be combined with a YUV inputFormat: the "
                      "converted frames are the library's, so the caller's buffers cannot serve as the history");
+        BGSB_REQUIRE(v == 0 || !c->gaussian_blur, "retainInput cannot be combined with gaussianBlur: the history is the "
+                     "blurred frame, so the caller's unblurred buffers cannot serve as it");
         c->retain_input = (v != 0);
+    }
+    else if (k == "gaussianBlur") {
+        BGSB_REQUIRE(v == 0 || v == 1, "gaussianBlur is 0 or 1");
+        BGSB_REQUIRE(v == 0 || !c->retain_input, "gaussianBlur cannot be combined with retainInput: the history is the "
+                     "blurred frame, so the caller's unblurred buffers cannot serve as it");
+        c->gaussian_blur = (int)v;
     }
     else if (k == "inputFormat") {
         BGSB_REQUIRE(v == BGSB_INPUT_BGR || v == BGSB_INPUT_NV12 || v == BGSB_INPUT_I420,
@@ -915,6 +952,7 @@ int bgsb_get_param(bgsb_ctx *c, const char *key, double *v)
     else if (k == "hostBands") *v = c->host_bands;
     else if (k == "retainInput") *v = c->retain_input;
     else if (k == "inputFormat") *v = c->input_format;
+    else if (k == "gaussianBlur") *v = c->gaussian_blur;
     else if (k == "quietGroups") *v = c->wmv_quiet;
     else if (k == "trace") *v = c->trace;
     else if (k == "ablTable") *v = c->abl_table;
@@ -997,11 +1035,23 @@ static int process_batch_impl(bgsb_ctx *c, const uint8_t *d_frames, int T, int w
         if (rc) return rc;
         d_frames = c->d_conv;
     }
+    const bool blur = c->gaussian_blur != 0;
+    if (blur) {          // likewise: all S x T frames blurred in one launch into a second scratch
+        const size_t need = (size_t)c->nstreams * T * c->npx * 3;
+        if (c->d_blur_bytes < need) {
+            cudaFree(c->d_blur); c->d_blur = nullptr; c->d_blur_bytes = 0;
+            BGSB_CUDA(cudaMalloc(&c->d_blur, need));
+            c->d_blur_bytes = need;
+        }
+        rc = blur_frames(d_frames, w, h, 0, h, c->nstreams * T, c->d_blur, (cudaStream_t)stream);
+        if (rc) return rc;
+        d_frames = c->d_blur;
+    }
     int64_t first = std::max<int64_t>(0, c->pi->warmup - c->nframes);
     if (first_fg_valid) *first_fg_valid = (int)std::min<int64_t>(first, T);
     const bool has_bg = c->pi->writes_bg;
     if (bg_valid) *bg_valid = has_bg && d_bg && (first < T);
-    if (c->retain_input && !yuv && c->pi->ring_history && (T == 1 || c->nstreams == 1)) {
+    if (c->retain_input && !yuv && !blur && c->pi->ring_history && (T == 1 || c->nstreams == 1)) {
         // "retainInput": the caller keeps the last one (FD) / two (WMV, WMM) frame buffers valid and unmodified, so
         // the history IS those buffers -- as in the host path's upload ring -- and nothing is written back:
         // FD moves its 7 algorithmic bytes per pixel, WMV its 10 (SURVEY 8d).
@@ -1046,6 +1096,9 @@ int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, u
     uint8_t *d_in = c->d_ring[c->ring_pos];
     const int fmt = c->input_format;       // YUV: the upload lands in d_yuv and is converted into the ring slot
     if (fmt != BGSB_INPUT_BGR && (rc = ensure_yuv_staging(c))) return rc;
+    const bool blur = c->gaussian_blur != 0;   // blur: the BGR frame lands in d_prep and is blurred into the ring slot
+    if (blur && (rc = ensure_prep_staging(c))) return rc;
+    uint8_t *const d_up = blur ? c->d_prep : d_in;
     const bool out_fg = mask_due(c), want_bg = bg_due(c, bg);
     // FD / WMV: history = the previous upload(s) in the ring -- no copy, the frame is read once
     const bool own_hist = !P.ring_history;
@@ -1062,10 +1115,14 @@ int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, u
     if (nchunks == 1) {
         mark(0, c->stream);
         if (fmt != BGSB_INPUT_BGR) BGSB_CUDA(upload_yuv(fmt, c->d_yuv, bgr, stride, w, h, 0, h, c->nstreams, c->stream));
-        else BGSB_CUDA(copy_rows(d_in, (size_t)w * 3, bgr, stride, (size_t)w * 3, rows, cudaMemcpyHostToDevice, c->stream));
+        else BGSB_CUDA(copy_rows(d_up, (size_t)w * 3, bgr, stride, (size_t)w * 3, rows, cudaMemcpyHostToDevice, c->stream));
         mark(1, c->stream); mark(2, c->stream);
         if (fmt != BGSB_INPUT_BGR) {
-            rc = convert_yuv(fmt, c->d_yuv, w, h, 0, h, c->nstreams, d_in, c->stream);
+            rc = convert_yuv(fmt, c->d_yuv, w, h, 0, h, c->nstreams, d_up, c->stream);
+            if (rc) return rc;
+        }
+        if (blur) {            // also on warm-up frames that launch no plugin kernel: the ring slot becomes history
+            rc = blur_frames(c->d_prep, w, h, 0, h, c->nstreams, d_in, c->stream);
             if (rc) return rc;
         }
         if (out_fg || P.warmup_launch) {
@@ -1081,19 +1138,32 @@ int bgsb_process(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, u
         mark(5, c->stream);
         BGSB_CUDA(cudaStreamSynchronize(c->stream));
     } else {
-        for (int i = 0; i < nchunks; i++) {
+        // band i arrives (upload, then the YUV conversion on the kernel stream), then band i's kernels run; with the blur
+        // they run one band later, because band i's blur reads up to 3 rows of band i + 1 (bands are >= 32 rows)
+        const int lag = blur ? 1 : 0;
+        for (int it = 0; it < nchunks + lag; it++) {
+            if (it < nchunks) {
+                const int r0 = it * band, nr = std::min(band, h - r0);
+                const size_t p0 = (size_t)r0 * w;
+                if (it == 0) mark(0, c->s_h2d);
+                if (fmt != BGSB_INPUT_BGR) BGSB_CUDA(upload_yuv(fmt, c->d_yuv, bgr, stride, w, h, r0, nr, 1, c->s_h2d));
+                else BGSB_CUDA(copy_rows(d_up + p0 * 3, (size_t)w * 3, bgr + (size_t)r0 * stride, stride, (size_t)w * 3, nr,
+                                         cudaMemcpyHostToDevice, c->s_h2d));
+                BGSB_CUDA(cudaEventRecord(c->ev_up[it], c->s_h2d));
+                if (it == nchunks - 1) mark(1, c->s_h2d);
+                BGSB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_up[it], 0));
+                if (it == 0) mark(2, c->stream);
+                if (fmt != BGSB_INPUT_BGR) {       // bands are multiples of 32 rows: whole chroma rows
+                    rc = convert_yuv(fmt, c->d_yuv, w, h, r0, nr, 1, d_up, c->stream);
+                    if (rc) return rc;
+                }
+            }
+            const int i = it - lag;
+            if (i < 0) continue;
             const int r0 = i * band, nr = std::min(band, h - r0);
             const size_t p0 = (size_t)r0 * w;
-            if (i == 0) mark(0, c->s_h2d);
-            if (fmt != BGSB_INPUT_BGR) BGSB_CUDA(upload_yuv(fmt, c->d_yuv, bgr, stride, w, h, r0, nr, 1, c->s_h2d));
-            else BGSB_CUDA(copy_rows(d_in + p0 * 3, (size_t)w * 3, bgr + (size_t)r0 * stride, stride, (size_t)w * 3, nr,
-                                     cudaMemcpyHostToDevice, c->s_h2d));
-            BGSB_CUDA(cudaEventRecord(c->ev_up[i], c->s_h2d));
-            if (i == nchunks - 1) mark(1, c->s_h2d);
-            BGSB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_up[i], 0));
-            if (i == 0) mark(2, c->stream);
-            if (fmt != BGSB_INPUT_BGR) {       // bands are multiples of 32 rows: whole chroma rows
-                rc = convert_yuv(fmt, c->d_yuv, w, h, r0, nr, 1, d_in, c->stream);
+            if (blur) {
+                rc = blur_frames(c->d_prep, w, h, r0, nr, 1, d_in, c->stream);
                 if (rc) return rc;
             }
             rc = launch_range(c, d_in, 1, c->d_fg, want_bg ? c->d_bg : nullptr, 0, own_hist, c->stream, p0, nr * w);
@@ -1168,15 +1238,22 @@ int bgsb_submit(bgsb_ctx *c, const uint8_t *bgr, int w, int h, size_t stride, ui
     uint8_t *o_fg = slot ? c->d_fg2 : c->d_fg, *o_bg = slot ? c->d_bg2 : c->d_bg;
     const int fmt = c->input_format;
     if (fmt != BGSB_INPUT_BGR && (rc = ensure_yuv_staging(c))) { drain(c); return rc; }
+    const bool blur = c->gaussian_blur != 0;
+    if (blur && (rc = ensure_prep_staging(c))) { drain(c); return rc; }
+    uint8_t *const d_up = blur ? c->d_prep : d_in;
 
-    // the input buffer (ring slot, or the YUV staging) was last read by the previous frame's kernels
+    // the input buffer (ring slot, or the YUV / blur staging) was last read by the previous frame's kernels
     if (c->seq > 0) BGSB_CUDA(cudaStreamWaitEvent(c->s_h2d, c->ev_k[slot ^ 1], 0));
     if (fmt != BGSB_INPUT_BGR) BGSB_CUDA(upload_yuv(fmt, c->d_yuv, bgr, stride, w, h, 0, h, c->nstreams, c->s_h2d));
-    else BGSB_CUDA(copy_rows(d_in, (size_t)w * 3, bgr, stride, (size_t)w * 3, rows, cudaMemcpyHostToDevice, c->s_h2d));
+    else BGSB_CUDA(copy_rows(d_up, (size_t)w * 3, bgr, stride, (size_t)w * 3, rows, cudaMemcpyHostToDevice, c->s_h2d));
     BGSB_CUDA(cudaEventRecord(c->ev_up[slot], c->s_h2d));
     BGSB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_up[slot], 0));
     if (fmt != BGSB_INPUT_BGR) {
-        rc = convert_yuv(fmt, c->d_yuv, w, h, 0, h, c->nstreams, d_in, c->stream);
+        rc = convert_yuv(fmt, c->d_yuv, w, h, 0, h, c->nstreams, d_up, c->stream);
+        if (rc) return rc;
+    }
+    if (blur) {
+        rc = blur_frames(c->d_prep, w, h, 0, h, c->nstreams, d_in, c->stream);
         if (rc) return rc;
     }
     if (out_fg || P.warmup_launch) {
@@ -1221,6 +1298,9 @@ int bgsb_process_fanout(bgsb_ctx *const *ctxs, int n, const uint8_t *bgr, int w,
     BGSB_REQUIRE(stride >= (size_t)w * (fmt == BGSB_INPUT_BGR ? 3 : 1), "stride smaller than a row");
     for (int k = 0; k < n; k++)
         BGSB_REQUIRE(ctxs[k]->input_format == fmt, "fan-out contexts must share one \"inputFormat\"");
+    const bool blur = c0->gaussian_blur != 0;  // blur: each band lands in c0's d_prep and is blurred once into the shared frame
+    for (int k = 0; k < n; k++)
+        BGSB_REQUIRE((ctxs[k]->gaussian_blur != 0) == blur, "fan-out contexts must share one \"gaussianBlur\"");
     for (int k = 0; k < n; k++) { if (int drc = drain(ctxs[k])) return drc; }
     for (int k = 0; k < n; k++) {
         BGSB_REQUIRE(ctxs[k] && fg[k], "null context or mask buffer");
@@ -1239,6 +1319,10 @@ int bgsb_process_fanout(bgsb_ctx *const *ctxs, int n, const uint8_t *bgr, int w,
         int rc = ensure_yuv_staging(c0);
         if (rc) return rc;
     }
+    if (blur) {
+        int rc = ensure_prep_staging(c0);
+        if (rc) return rc;
+    }
     const size_t fbytes = (size_t)w * h * 3;
     if (c0->d_fan_bytes < fbytes) {
         cudaFree(c0->d_fan); c0->d_fan = nullptr; c0->d_fan_bytes = 0;
@@ -1254,16 +1338,28 @@ int bgsb_process_fanout(bgsb_ctx *const *ctxs, int n, const uint8_t *bgr, int w,
         fgv[k] = mask_due(ctxs[k]);
         bgv[k] = bg_due(ctxs[k], bg ? bg[k] : nullptr);
     }
-    for (int i = 0; i < nchunks; i++) {
+    uint8_t *const d_up = blur ? c0->d_prep : c0->d_fan;
+    const int lag = blur ? 1 : 0;        // band i's blur reads up to 3 rows of band i + 1, as in bgsb_process
+    for (int it = 0; it < nchunks + lag; it++) {
+        if (it < nchunks) {
+            const int r0 = it * band, nr = std::min(band, h - r0);
+            const size_t p0 = (size_t)r0 * w;
+            if (fmt != BGSB_INPUT_BGR) {
+                BGSB_CUDA(upload_yuv(fmt, c0->d_yuv, bgr, stride, w, h, r0, nr, 1, c0->s_h2d));
+                int rc = convert_yuv(fmt, c0->d_yuv, w, h, r0, nr, 1, d_up, c0->s_h2d);
+                if (rc) return rc;
+            } else {
+                BGSB_CUDA(copy_rows(d_up + p0 * 3, (size_t)w * 3, bgr + (size_t)r0 * stride, stride, (size_t)w * 3, nr,
+                                    cudaMemcpyHostToDevice, c0->s_h2d));
+            }
+        }
+        const int i = it - lag;
+        if (i < 0) continue;
         const int r0 = i * band, nr = std::min(band, h - r0);
         const size_t p0 = (size_t)r0 * w;
-        if (fmt != BGSB_INPUT_BGR) {
-            BGSB_CUDA(upload_yuv(fmt, c0->d_yuv, bgr, stride, w, h, r0, nr, 1, c0->s_h2d));
-            int rc = convert_yuv(fmt, c0->d_yuv, w, h, r0, nr, 1, c0->d_fan, c0->s_h2d);
+        if (blur) {
+            int rc = blur_frames(c0->d_prep, w, h, r0, nr, 1, c0->d_fan, c0->s_h2d);
             if (rc) return rc;
-        } else {
-            BGSB_CUDA(copy_rows(c0->d_fan + p0 * 3, (size_t)w * 3, bgr + (size_t)r0 * stride, stride, (size_t)w * 3, nr,
-                                cudaMemcpyHostToDevice, c0->s_h2d));
         }
         BGSB_CUDA(cudaEventRecord(c0->ev_up[i], c0->s_h2d));
         for (int k = 0; k < n; k++) {

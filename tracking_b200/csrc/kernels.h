@@ -205,6 +205,17 @@ struct Yuv420Launch {
 };
 int launch_yuv420_to_bgr(const Yuv420Launch &L, cudaStream_t stream);
 
+// ---- pre-processing: cv::GaussianBlur(Size(7, 7), 1.5) of dense BGR frames, the PreProcessor's gaussianBlur (prep/gauss7.cu) ----
+struct Gauss7Launch {
+    const uint8_t *src;      // [nframes][h][w][3], frames frame_stride bytes apart
+    uint8_t *dst;            // the same layout; may not overlap src
+    size_t frame_stride;
+    int w, h;                // the whole frame: taps reflect at its edges
+    int r0, nr;              // output rows [r0, r0 + nr); rows r0 - 3 .. r0 + nr + 2 (reflected) are read
+    int nframes;
+};
+int launch_gauss7(const Gauss7Launch &L, cudaStream_t stream);
+
 // ---- synthetic video ----------------------------------------------------------------------------
 int launch_synth(uint8_t *d_frames, int nstreams, int T, int w, int h, int t0, uint32_t seed0,
                  cudaStream_t stream);
